@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the CLSuperPathTracer hot path (BASELINE.json metric: Mrays/s and samples/s per image).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one image: render the workload's frame (all samples of all pixels)
 into device memory.  BASELINE.json quotes its metric on no single config, so the defaults are
@@ -32,6 +32,13 @@ into device memory.  BASELINE.json quotes its metric on no single config, so the
   cpu_baseline: the reference's own CPU run of the same frame (oracle/_ref = unmodified reference compiled through
             oracle/refrt) where it can hold the workload (<= 512 triangles, 64 spp), else the C oracle port on rows
             sampled over the frame, all host cores, thread count verified.
+  --impl reference : that CPU measurement alone, once per warm-up and timed step; each step costs about --cpu-budget
+            seconds of CPU work (whole light frames: their full reference run), so the run grows with --steps.
+  step_ms : the time of every timed step; `steps` is their count.
+  --dump-outputs DIR : after the timed steps of the headline workload, what its last step left for the caller is written as
+            DIR/<name>.npy in float32: image.npy = the (H, W, 4) RGBA8 frame, and at N > 1 accum.npy = the reduced float
+            accumulation buffer.  Inputs are fixed (seeds, scene, synthetic mesh seed), so two builds can be compared file for
+            file.  Above 64 MB in all, every array keeps the same seeded sample of rows, listed in rows.npy (float64).
 """
 import argparse
 import hashlib
@@ -380,8 +387,9 @@ def bench_reference(args, w, wname):
     msamples = sum(m["msamples"] for m in runs) / len(runs)
     kind, cores, sample = runs[0]["kind"], runs[0]["cores"], runs[0]["sample"]
     line = {
-        "impl": "reference", "metric": "Mrays/s", "value": mrays, "unit": "Mrays/s", "n_gpus": args.gpus, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "strong" if (strong and world > 1) else "weak",
+        "impl": "reference", "metric": "Mrays/s", "value": mrays, "unit": "Mrays/s", "n_gpus": args.gpus, "steps": len(runs),
+        "warmup": args.warmup, "ms_per_step": ms, "step_ms": [round(m["ms"], 3) for m in runs], "higher_is_better": True,
+        "scaling": "strong" if (strong and world > 1) else "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": workload_config(w, wname, W, H, spp),
         "msamples_per_s": msamples, "rays_per_step": runs[0]["rays"], "samples_per_step": runs[0]["samples"],
@@ -430,6 +438,27 @@ def check_against_oracle(w, d, W, H, spp, image, rerender=None, extra=None):
             "oracle_s": round(time.perf_counter() - t0, 2)}
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+DUMP_ROW_SEED = 20261018
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every (H, ...) array of `arrays` as out_dir/<name>.npy in float32 (RGBA8 values are exact in it).  When they
+    exceed DUMP_LIMIT_BYTES in all, each keeps the same fixed, seeded sample of rows, written as rows.npy (float64)."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v, np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        H = next(iter(arrays.values())).shape[0]
+        keep = max(1, H * (DUMP_LIMIT_BYTES - (1 << 20)) // total)      # 1 MiB left for the row list and the .npy headers
+        rows = np.sort(np.random.default_rng(DUMP_ROW_SEED).choice(H, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------- our arm
 class Ours:
     def __init__(self, args):
@@ -444,6 +473,7 @@ class Ours:
         torch.cuda.set_device(self.local_rank)
         self.dist = None
         self.saved_stdout = None
+        self.outputs = None                          # rank 0, headline workload: what the last timed step computed
         if self.world > 1:
             # NCCL (NCCL_DEBUG=INFO/VERSION) prints on stdout; the contract is ONE JSON line there -> park stdout on stderr
             # for the duration of the run (NCCL_DEBUG itself is left exactly as the caller set it)
@@ -573,6 +603,10 @@ class Ours:
         if world > 1:
             dist.barrier()
         clocks = sampler.finish(t0, t1) if sampler else None
+        if headline and args.dump_outputs and rank == 0:
+            self.outputs = {"image": rgba.cpu().numpy().view(np.uint8).reshape(H, W, 4)}
+            if accum is not None:                    # rank 0 holds the reduced sum
+                self.outputs["accum"] = accum.cpu().numpy()
         step_ms = [s.elapsed_time(e) for s, e in zip(starts, stops)]
         total_ms = sum(step_ms)
         rays, samples, rays_traced = float(counters_ref["rays"]), float(counters_ref["samples"]), float(counters["rays"])
@@ -714,8 +748,8 @@ class Ours:
             if ncu.get("warp_instructions"):
                 roof["issue_frac"] = ncu["warp_instructions"] / (kernel_ms * 1e-3) / 1e9 / issue_peak
         line = {
-            "metric": "Mrays/s", "value": rays / 1e3 / ms_per_step, "unit": "Mrays/s", "n_gpus": world, "steps": steps,
-            "warmup": warm, "ms_per_step": ms_per_step, "higher_is_better": True,
+            "metric": "Mrays/s", "value": rays / 1e3 / ms_per_step, "unit": "Mrays/s", "n_gpus": world, "steps": len(step_ms),
+            "warmup": warm, "ms_per_step": ms_per_step, "step_ms": [round(x, 4) for x in step_ms], "higher_is_better": True,
             "scaling": ("strong" if strong else "weak") if world > 1 else "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": dict(workload_config(w, wname, W, H, spp), kernel=args.kernel, kernel_resolved=resolved_kernel, scene_mem=args.scene_mem or "auto",
@@ -757,6 +791,8 @@ class Ours:
 def bench_ours(args, wname, default_workload):
     b = Ours(args)
     line = b.measure(wname, args.steps, args.warmup, headline=True)
+    if b.outputs is not None:
+        dump_outputs(args.dump_outputs, b.outputs)
     ok = True
     if b.rank == 0:
         if b.world == 1 and default_workload and not args.no_extras:
@@ -794,7 +830,8 @@ def bench_ours(args, wname, default_workload):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps; with --impl reference each step is about --cpu-budget seconds of CPU work")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=None, choices=sorted(WORKLOADS),
@@ -813,15 +850,19 @@ def main():
                          "samples (throughput mode, statistically equivalent)")
     ap.add_argument("--strong", action="store_true", help="(default at N>1) keep the image fixed as N grows")
     ap.add_argument("--weak", action="store_true", help="N>1: grow the image with N (512 x 512N style) instead of strong scaling")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload computed as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times CPU rows, not a frame")
     world = max(1, args.gpus, int(os.environ.get("WORLD_SIZE", "1")))
     default_workload = args.workload is None
     wname = args.workload or (DEFAULT_N1 if world == 1 else DEFAULT_MULTI)
     if args.impl == "reference":
         # the CPU arm must use every host core whatever the launcher exported (torchrun sets OMP_NUM_THREADS=1)
         os.environ["OMP_NUM_THREADS"] = str(host_cores())
-        if args.steps > 3:
-            args.steps = 3       # each step is ~cpu-budget seconds of CPU work; keep the whole run within minutes
         args.warmup = min(args.warmup, 1)
         bench_reference(args, WORKLOADS[wname], wname)
     else:

@@ -53,6 +53,46 @@ def test_reference_arm_light_workload_runs_the_unmodified_reference_binary():
     assert j["cpu_baseline"]["kind"] == "reference" and "%d OpenMP threads" % len(os.sched_getaffinity(0)) in j["cpu_baseline"]["sample"]
 
 
+def test_reference_arm_runs_the_requested_number_of_steps():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "4", "--warmup", "0",
+                        "--cpu-budget", "0.2", "--workload", "nodof_512x512x64"], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert p.returncode == 0, p.stderr[-2000:]
+    j = json.loads(p.stdout.strip())
+    assert j["steps"] == 4 and len(j["step_ms"]) == 4 and all(ms > 0 for ms in j["step_ms"])
+    assert abs(j["ms_per_step"] - sum(j["step_ms"]) / 4) < 1e-2
+
+
+def test_bench_refuses_zero_steps_and_dumps_of_the_reference_arm(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "out")]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert p.returncode == 2 and p.stdout == "" and "error" in p.stderr, extra
+    assert not os.path.exists(tmp_path / "out")
+
+
+def test_dump_outputs_keeps_whole_arrays_below_the_limit_and_the_same_seeded_rows_above_it(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(1)
+    img = rng.integers(0, 256, (1024, 256, 4), dtype=np.uint8)
+    acc = rng.random((1024, 256, 4), dtype=np.float32)
+    bench.dump_outputs(str(tmp_path / "whole"), {"image": img})
+    assert sorted(os.listdir(tmp_path / "whole")) == ["image.npy"]
+    got = np.load(tmp_path / "whole" / "image.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, img)
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 3 << 20)         # image + accum as float32: 8 MiB
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"image": img, "accum": acc})
+    d = tmp_path / "a"
+    assert sorted(os.listdir(d)) == ["accum.npy", "image.npy", "rows.npy"]
+    assert sum(os.path.getsize(d / f) for f in os.listdir(d)) <= 3 << 20
+    rows = np.load(d / "rows.npy")
+    assert rows.dtype == np.float64 and len(rows) > 100 and np.all(np.diff(rows) > 0)
+    r = rows.astype(np.int64)
+    assert np.array_equal(np.load(d / "image.npy"), img[r]) and np.array_equal(np.load(d / "accum.npy"), acc[r])
+    for f in os.listdir(d):
+        assert (d / f).read_bytes() == (tmp_path / "b" / f).read_bytes(), f
+
+
 def test_reference_arm_other_ranks_stay_silent():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],

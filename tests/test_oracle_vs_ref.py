@@ -9,7 +9,9 @@ import pytest
 from conftest import REF_BUILD, REFERENCE, SEED_SETS
 
 pytestmark = pytest.mark.needs_reference
-have_ref = os.path.isdir(REFERENCE) and os.path.exists(os.path.join(REF_BUILD, "bin", "base", "CLSuperPathTracer"))
+have_ref = all(os.path.exists(os.path.join(REF_BUILD, "bin", v, e)) for v, e in
+               (("base", "CLSuperPathTracer"), ("lmem", "CLSuperPathTracer"), ("nodof", "CLSuperPathTracer"), ("grid", "CLSuperPathTracer"),
+                ("bidir", "CLSuperBidirectionalPathTracer")))
 
 
 @pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="needs /root/reference")
