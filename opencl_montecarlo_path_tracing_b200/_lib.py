@@ -143,6 +143,7 @@ PTCUDA_SYMBOLS = {
     "pt_release_event": (None, [_VP]),
     "pt_synchronize": (_I, [_VP]),
     "pt_probe_trace": (_I, [_VP, _I, _I, _I, _FP, _FP, _FP, _I32P, _FP]),
+    "pt_probe_trace_counts": (_I, [_VP, _I, _I, _I, _FP, _FP, _FP, _I32P, _FP, _U32P, _U32P]),
     "pt_selftest_fastmath": (_I, [_VP, C.c_uint64, C.c_uint32, C.POINTER(C.c_uint64)]),
     "pt_probe_rng": (_I, [_VP, _U32P, C.c_uint32, _I, _FP, _U32P]),
     "pt_measure_peaks": (_I, [_VP, C.POINTER(C.c_double)]),

@@ -393,18 +393,25 @@ class Renderer:
     def synchronize(self):
         _check(self._l.pt_synchronize(self.ctx), "pt_synchronize")
 
-    def probe_trace(self, variant, origins, dirs, t_in, arith="fma"):
-        o = np.ascontiguousarray(origins, np.float32)
-        d = np.ascontiguousarray(dirs, np.float32)
-        t = np.ascontiguousarray(t_in, np.float32).copy()
+    def probe_trace(self, variant, origins, dirs, t_in, arith="fma", counts=False):
+        """Device TraceRay on single rays -> (material, t, normal), plus (cells visited, triangle tests) with counts=True
+        (include/ptcuda.h pt_probe_trace_counts)."""
+        o = np.ascontiguousarray(origins, np.float32).reshape(-1, 3)
+        d = np.ascontiguousarray(dirs, np.float32).reshape(-1, 3)
+        t = np.ascontiguousarray(t_in, np.float32).reshape(-1).copy()
         n = o.shape[0]
+        if d.shape[0] != n or t.shape[0] != n:
+            raise ValueError("probe_trace: origins, dirs and t_in must describe the same number of rays")
         m = np.zeros(n, np.int32)
         nrm = np.zeros((n, 3), np.float32)
-        fp = C.POINTER(C.c_float)
-        _check(self._l.pt_probe_trace(self.ctx, PT_VARIANT[variant], PT_ARITH[arith], n, o.ctypes.data_as(fp), d.ctypes.data_as(fp),
-                                      t.ctypes.data_as(fp), m.ctypes.data_as(C.POINTER(C.c_int32)), nrm.ctypes.data_as(fp)),
+        cells = np.zeros(n, np.uint32)
+        tests = np.zeros(n, np.uint32)
+        fp, up = C.POINTER(C.c_float), C.POINTER(C.c_uint32)
+        _check(self._l.pt_probe_trace_counts(self.ctx, PT_VARIANT[variant], PT_ARITH[arith], n, o.ctypes.data_as(fp),
+                                             d.ctypes.data_as(fp), t.ctypes.data_as(fp), m.ctypes.data_as(C.POINTER(C.c_int32)),
+                                             nrm.ctypes.data_as(fp), cells.ctypes.data_as(up), tests.ctypes.data_as(up)),
                "pt_probe_trace")
-        return m, t, nrm
+        return (m, t, nrm, cells, tests) if counts else (m, t, nrm)
 
     def selftest_fastmath(self, npairs, seed=1):
         out = (C.c_uint64 * 3)()

@@ -1027,8 +1027,8 @@ __global__ void k_tonemap(const float4 *__restrict__ accum, uint32_t *__restrict
 }
 
 template <bool FMA>
-__global__ void k_probe_trace(int variant, int n, const float *o, const float *d, float *t, int *m, float *nrm,
-                              const __grid_constant__ LaunchArgs P) {
+__global__ void k_probe_trace(int variant, int n, const float *o, const float *d, float *t, int *m, float *nrm, uint32_t *cells,
+                              uint32_t *tests, const __grid_constant__ LaunchArgs P) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     V3 oo = mk3(o[3 * i], o[3 * i + 1], o[3 * i + 2]), dd = mk3(d[3 * i], d[3 * i + 1], d[3 * i + 2]);
@@ -1048,6 +1048,8 @@ __global__ void k_probe_trace(int variant, int n, const float *o, const float *d
     }
     t[i] = tt; m[i] = hit_material(hit);
     nrm[3 * i] = nn.x; nrm[3 * i + 1] = nn.y; nrm[3 * i + 2] = nn.z;
+    cells[i] = cnt.cells;
+    tests[i] = variant == PT_VARIANT_GRID ? cnt.gtri : cnt.btests;
 }
 
 __global__ void k_probe_rng(uint4 seeds, uint32_t gid, int nsteps, float *out_f, uint32_t *out_state) {
@@ -1064,23 +1066,28 @@ extern "C" int pt_tonemap_device(pt_ctx c, const void *d_accum, void *d_rgba8, i
     return 0;
 }
 
-extern "C" int pt_probe_trace(pt_ctx c, int variant, int arith, int n, const float *o, const float *d, float *t_inout,
-                              int32_t *m_out, float *n_out) {
+extern "C" int pt_probe_trace_counts(pt_ctx c, int variant, int arith, int n, const float *o, const float *d, float *t_inout,
+                                     int32_t *m_out, float *n_out, uint32_t *cells_out, uint32_t *tests_out) {
     if (!c->scene_set) return pt_fail(1, "pt_probe_trace: no scene");
     if (variant == PT_VARIANT_GRID && !c->grid_set) return pt_fail(1, "pt_probe_trace: no grid");
+    if (n < 0) return pt_fail(1, "pt_probe_trace: n < 0");
+    if (n == 0) return 0;
     PT_CUDA(cudaSetDevice(c->device), "select device");
     const int ar = arith != PT_ARITH_SEPARATE ? PT_ARITH_FMA : PT_ARITH_SEPARATE;
     DevLock lock(c->device);
     int rc = pt_bind_const_scene(c, ar);
     if (rc) return rc;
+    const size_t nn = (size_t)n;
     float *d_o, *d_d, *d_t, *d_n;
     int *d_m;
-    PT_CUDA(cudaMalloc(&d_o, n * 12), "alloc"); PT_CUDA(cudaMalloc(&d_d, n * 12), "alloc");
-    PT_CUDA(cudaMalloc(&d_t, n * 4), "alloc"); PT_CUDA(cudaMalloc(&d_n, n * 12), "alloc");
-    PT_CUDA(cudaMalloc(&d_m, n * 4), "alloc");
-    cudaMemcpyAsync(d_o, o, n * 12, cudaMemcpyHostToDevice, c->stream);
-    cudaMemcpyAsync(d_d, d, n * 12, cudaMemcpyHostToDevice, c->stream);
-    cudaMemcpyAsync(d_t, t_inout, n * 4, cudaMemcpyHostToDevice, c->stream);
+    uint32_t *d_cells, *d_tests;
+    PT_CUDA(cudaMalloc(&d_o, nn * 12), "alloc"); PT_CUDA(cudaMalloc(&d_d, nn * 12), "alloc");
+    PT_CUDA(cudaMalloc(&d_t, nn * 4), "alloc"); PT_CUDA(cudaMalloc(&d_n, nn * 12), "alloc");
+    PT_CUDA(cudaMalloc(&d_m, nn * 4), "alloc");
+    PT_CUDA(cudaMalloc(&d_cells, nn * 4), "alloc"); PT_CUDA(cudaMalloc(&d_tests, nn * 4), "alloc");
+    cudaMemcpyAsync(d_o, o, nn * 12, cudaMemcpyHostToDevice, c->stream);
+    cudaMemcpyAsync(d_d, d, nn * 12, cudaMemcpyHostToDevice, c->stream);
+    cudaMemcpyAsync(d_t, t_inout, nn * 4, cudaMemcpyHostToDevice, c->stream);
     pt_camera cam0;
     memset(&cam0, 0, sizeof(cam0));
     pt_render_params rp0;
@@ -1088,15 +1095,24 @@ extern "C" int pt_probe_trace(pt_ctx c, int variant, int arith, int n, const flo
     rp0.variant = variant; rp0.width = 1; rp0.height = 1; rp0.spp = 64; rp0.arith = ar;
     pt::LaunchArgs LA;
     fill_args(c, &cam0, &rp0, nullptr, nullptr, nullptr, &LA);
-    if (ar == PT_ARITH_FMA) pt::k_probe_trace<true><<<(n + 127) / 128, 128, 0, c->stream>>>(variant, n, d_o, d_d, d_t, d_m, d_n, LA);
-    else pt::k_probe_trace<false><<<(n + 127) / 128, 128, 0, c->stream>>>(variant, n, d_o, d_d, d_t, d_m, d_n, LA);
+    if (ar == PT_ARITH_FMA)
+        pt::k_probe_trace<true><<<(n + 127) / 128, 128, 0, c->stream>>>(variant, n, d_o, d_d, d_t, d_m, d_n, d_cells, d_tests, LA);
+    else
+        pt::k_probe_trace<false><<<(n + 127) / 128, 128, 0, c->stream>>>(variant, n, d_o, d_d, d_t, d_m, d_n, d_cells, d_tests, LA);
     PT_CUDA(cudaGetLastError(), "probe trace");
-    cudaMemcpyAsync(t_inout, d_t, n * 4, cudaMemcpyDeviceToHost, c->stream);
-    cudaMemcpyAsync(m_out, d_m, n * 4, cudaMemcpyDeviceToHost, c->stream);
-    cudaMemcpyAsync(n_out, d_n, n * 12, cudaMemcpyDeviceToHost, c->stream);
+    cudaMemcpyAsync(t_inout, d_t, nn * 4, cudaMemcpyDeviceToHost, c->stream);
+    if (m_out) cudaMemcpyAsync(m_out, d_m, nn * 4, cudaMemcpyDeviceToHost, c->stream);
+    if (n_out) cudaMemcpyAsync(n_out, d_n, nn * 12, cudaMemcpyDeviceToHost, c->stream);
+    if (cells_out) cudaMemcpyAsync(cells_out, d_cells, nn * 4, cudaMemcpyDeviceToHost, c->stream);
+    if (tests_out) cudaMemcpyAsync(tests_out, d_tests, nn * 4, cudaMemcpyDeviceToHost, c->stream);
     PT_CUDA(cudaStreamSynchronize(c->stream), "sync probe");
-    cudaFree(d_o); cudaFree(d_d); cudaFree(d_t); cudaFree(d_n); cudaFree(d_m);
+    cudaFree(d_o); cudaFree(d_d); cudaFree(d_t); cudaFree(d_n); cudaFree(d_m); cudaFree(d_cells); cudaFree(d_tests);
     return 0;
+}
+
+extern "C" int pt_probe_trace(pt_ctx c, int variant, int arith, int n, const float *o, const float *d, float *t_inout,
+                              int32_t *m_out, float *n_out) {
+    return pt_probe_trace_counts(c, variant, arith, n, o, d, t_inout, m_out, n_out, nullptr, nullptr);
 }
 
 extern "C" int pt_selftest_fastmath(pt_ctx c, uint64_t npairs, uint32_t seed, uint64_t out[3]) {

@@ -372,6 +372,9 @@ static inline void camera_ray(const oracle_job *J, Rng *rng, int i, int j, V3 *o
     *d = normalize3(vmadd(A, 16.0f, nd));
 }
 
+/* the grid of a trianglegrid job is given (the CSR arrays; refs may be absent only without triangles) */
+static int grid_job_ok(const oracle_job *J) { return J->cell_start && (J->cell_refs || J->ntriangles <= 0); }
+
 static void scene_from_job(const oracle_job *J, Scene *S) {
     memset(S, 0, sizeof(*S));
     S->carry = J->variant != ORACLE_BASE;
@@ -651,7 +654,7 @@ int oracle_render(const oracle_job *J, uint8_t *rgba8, float *accum, uint32_t *r
     if ((J->variant == ORACLE_BIDIR || J->variant == ORACLE_VLPGRID) && (J->nvpl < 0 || (J->nvpl > 0 && !J->vpls))) return -1;
     if (J->variant == ORACLE_VLPGRID && (!J->cell_start || !J->cell_refs)) return -1;
     if (J->variant == ORACLE_NODOF && J->spp != 64) return -1;
-    if (J->variant == ORACLE_GRID && (!J->cell_start || (!J->cell_refs && J->ntriangles > 0))) return -1;
+    if (J->variant == ORACLE_GRID && !grid_job_ok(J)) return -1;
     Scene S;
     scene_from_job(J, &S);
     const int W = J->width, H = J->height;
@@ -738,6 +741,28 @@ int oracle_render(const oracle_job *J, uint8_t *rgba8, float *accum, uint32_t *r
         cnt_add(&total, &cnt);
     }
     if (counters) *counters = total;
+    return 0;
+}
+
+int oracle_trace_rays(const oracle_job *J, int n, const float *o, const float *d, float *t_inout, int32_t *m_out,
+                      float *n_out, uint32_t *cells_out, uint32_t *tests_out) {
+    if (!J || n < 0 || (n > 0 && (!o || !d || !t_inout)) || J->variant < 0 || J->variant > 5) return -1;
+    if (J->variant == ORACLE_GRID && !grid_job_ok(J)) return -1;
+    oracle_job Jr = *J;
+    if (Jr.variant != ORACLE_BASE && Jr.variant != ORACLE_GRID) Jr.variant = ORACLE_LMEM;   /* lmem TraceRay semantics */
+    Scene S;
+    scene_from_job(&Jr, &S);
+    for (int k = 0; k < n; ++k) {
+        oracle_counters cnt;
+        memset(&cnt, 0, sizeof(cnt));
+        V3 nn = v3(0, 0, 0);
+        const int m = trace_ray(&S, v3(o[3 * k], o[3 * k + 1], o[3 * k + 2]), v3(d[3 * k], d[3 * k + 1], d[3 * k + 2]),
+                                t_inout + k, &nn, &cnt);
+        if (m_out) m_out[k] = m;
+        if (n_out) { n_out[3 * k] = nn.x; n_out[3 * k + 1] = nn.y; n_out[3 * k + 2] = nn.z; }
+        if (cells_out) cells_out[k] = (uint32_t)cnt.cells_visited;
+        if (tests_out) tests_out[k] = (uint32_t)cnt.tri_tests;
+    }
     return 0;
 }
 

@@ -115,6 +115,12 @@ uint32_t oracle_randomize_id(uint32_t id);
 /* Single-ray probe of TraceRay for brute-force variants (carry = 0: base semantics, 1: lmem). */
 int oracle_trace_ray(int carry, const float o[3], const float d[3], float *t_inout, float n_out[3],
                      const int32_t spheres[9], const int32_t squares[9], const float *tris12, int ntris);
+/* TraceRay on n rays (o, d: n x 3 floats) with the scene of `job`: job->variant ORACLE_BASE (t reset per call), ORACLE_GRID
+ * (triangles through job's uniform grid, set up as for oracle_render) or any other (lmem semantics, brute force).  t_inout is
+ * each ray's carried hit bound and receives its final t.  Optional outputs per ray: material m_out, normal n_out (n x 3, zero
+ * on a miss), grid cells the walk visited (cells_out) and Moller-Trumbore tests started (tests_out).  0, or -1 on bad arguments. */
+int oracle_trace_rays(const oracle_job *job, int n, const float *o, const float *d, float *t_inout, int32_t *m_out,
+                      float *n_out, uint32_t *cells_out, uint32_t *tests_out);
 
 /* ---- host-side restatements (oracle_host.c) ---- */
 /* CLSuperPathTracer.c:236-243 */

@@ -72,6 +72,8 @@ class OracleLib:
         L.oracle_randomize_id.argtypes = [C.c_uint32]
         L.oracle_build_grid.restype = C.c_uint64
         L.oracle_trace_ray.restype = C.c_int
+        L.oracle_trace_rays.restype = C.c_int
+        L.oracle_trace_rays.argtypes = [C.POINTER(oracle_job), C.c_int] + [C.c_void_p] * 7
         L.oracle_save_pam.restype = C.c_int
         L.oracle_save_pam.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p]
         assert L.oracle_contract_mode() == self.contract
@@ -186,6 +188,52 @@ class OracleLib:
                 J.lights[i][k] = float(lights[i, k])
         return tris
 
+    def _fill_grid(self, J, tris, scene, grid, modifier):
+        """Triangle grid part of an oracle_job.  `grid`: {"box_min", "box_max", "res", "cell_size"[, "csr"]}; None sizes it as the
+        reference host does (scene box, CELL_SIZE_MODIFIER `modifier`).  The binning is stored back into `grid` as "csr", so
+        callers that keep `grid` reuse it.  Returns the arrays that must stay alive while J is used."""
+        if grid is None:
+            res, cell = self.grid_dims(scene["box_min"], scene["box_max"], tris.shape[0], modifier)
+            grid = {"box_min": scene["box_min"], "box_max": scene["box_max"], "res": res, "cell_size": cell}
+        if "csr" in grid:
+            start, refs = grid["csr"]
+        else:
+            start, refs = self.build_grid(tris, grid["box_min"], grid["res"], grid["cell_size"])
+            grid["csr"] = (start, refs)
+        if refs.size == 0:
+            refs = np.zeros(1, np.uint32)
+        J.box_min[:] = [float(x) for x in grid["box_min"]]; J.box_max[:] = [float(x) for x in grid["box_max"]]
+        J.grid_res[:] = [int(x) for x in grid["res"]]; J.cell_size[:] = [float(x) for x in grid["cell_size"]]
+        J.cell_start = start.ctypes.data_as(C.POINTER(C.c_uint32))
+        J.cell_refs = refs.ctypes.data_as(C.POINTER(C.c_uint32))
+        return start, refs
+
+    def trace_rays(self, variant, origins, dirs, t_in, scene, grid=None, modifier=3.0):
+        """TraceRay on single rays (oracle_trace_rays): variant "base" (t reset per call), "lmem" (carried t) or "grid"
+        (lmem semantics, triangles through the uniform grid; `grid` as for render).  -> dict of material, t, normal,
+        cells (grid cells visited) and tests (Moller-Trumbore tests started), one entry per ray."""
+        J = oracle_job()
+        J.variant = VARIANTS[variant]
+        tris = self._fill_scene(J, (0, 0, 0, 0), scene)
+        keep = self._fill_grid(J, tris, scene, grid, modifier) if variant == "grid" else None
+        o = np.ascontiguousarray(origins, np.float32).reshape(-1, 3)
+        d = np.ascontiguousarray(dirs, np.float32).reshape(-1, 3)
+        t = np.ascontiguousarray(t_in, np.float32).reshape(-1).copy()
+        n = o.shape[0]
+        if d.shape[0] != n or t.shape[0] != n:
+            raise ValueError("trace_rays: origins, dirs and t_in must describe the same number of rays")
+        m = np.zeros(n, np.int32)
+        nrm = np.zeros((n, 3), np.float32)
+        cells = np.zeros(n, np.uint32)
+        tests = np.zeros(n, np.uint32)
+        vp = C.c_void_p
+        rc = self.lib.oracle_trace_rays(C.byref(J), int(n), o.ctypes.data_as(vp), d.ctypes.data_as(vp), t.ctypes.data_as(vp),
+                                        m.ctypes.data_as(vp), nrm.ctypes.data_as(vp), cells.ctypes.data_as(vp), tests.ctypes.data_as(vp))
+        del tris, keep
+        if rc:
+            raise ValueError("oracle_trace_rays rejected the job")
+        return {"m": m, "t": t, "n": nrm, "cells": cells, "tests": tests}
+
     def light_tracer(self, seeds, scene, n_vlp=512, want_rng=False):
         """Kernel lightTracer (bidirectionalpathtracer.ocl:280-326): -> (n_vlp*nlights, 4) float32 VPL buffer."""
         J = oracle_job()
@@ -260,21 +308,7 @@ class OracleLib:
             J.cell_start = start.ctypes.data_as(C.POINTER(C.c_uint32))
             J.cell_refs = refs.ctypes.data_as(C.POINTER(C.c_uint32))
         if variant == "grid":
-            if grid is None:
-                res, cell = self.grid_dims(scene["box_min"], scene["box_max"], tris.shape[0], modifier)
-                grid = {"box_min": scene["box_min"], "box_max": scene["box_max"], "res": res, "cell_size": cell}
-            if "csr" in grid:
-                start, refs = grid["csr"]
-            else:
-                start, refs = self.build_grid(tris, grid["box_min"], grid["res"], grid["cell_size"])
-                grid["csr"] = (start, refs)          # callers that keep `grid` reuse the binning
-            if refs.size == 0:
-                refs = np.zeros(1, np.uint32)
-            keep = (start, refs)
-            J.box_min[:] = [float(x) for x in grid["box_min"]]; J.box_max[:] = [float(x) for x in grid["box_max"]]
-            J.grid_res[:] = [int(x) for x in grid["res"]]; J.cell_size[:] = [float(x) for x in grid["cell_size"]]
-            J.cell_start = start.ctypes.data_as(C.POINTER(C.c_uint32))
-            J.cell_refs = refs.ctypes.data_as(C.POINTER(C.c_uint32))
+            keep = self._fill_grid(J, tris, scene, grid, modifier)
         J.nthreads = nthreads
         img = np.zeros((height, width, 4), np.uint8)
         acc = np.zeros((height, width, 4), np.float32) if want_accum else None

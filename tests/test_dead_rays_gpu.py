@@ -30,10 +30,12 @@ def _same_bits(res, ref, rows, W, H, what):
 
 @pytest.mark.parametrize("variant,mesh", [("base", "base"), ("lmem", "lmem"), ("grid", "grid"), ("base", "torus")])
 @pytest.mark.parametrize("arith", ["fma", "separate"])
-@pytest.mark.parametrize("kernel", ["auto", "mega", "spec"])
+@pytest.mark.parametrize("kernel", ["auto", "mega", "spec", "grid_queue", "grid_async"])
 def test_elided_frames_keep_every_bit(renderer, scene_dirs, oracle_fma, oracle_sep, variant, mesh, arith, kernel):
     if kernel == "spec" and variant == "grid":
         pytest.skip("PT_KERNEL_SPEC is for the brute-force variants")
+    if kernel.startswith("grid_") and variant != "grid":
+        pytest.skip("%s is a trianglegrid kernel" % kernel)
     o = oracle_fma if arith == "fma" else oracle_sep
     d = scene_dirs[mesh]
     scene = pt.load_scene_dir(d, variant)
@@ -105,6 +107,30 @@ def test_soup1m_config4_window_elided(oracle_fma):
             _same_bits(el, ref, rows, W, H, "config 4 rows %s elide" % (rows,))
             assert el.counters["rays"] < ref["counters"]["rays"]
             assert el.counters["cells_visited"] < ref["counters"]["cells_visited"]
+
+
+def test_config4_window_trace_and_elide_legs():
+    """config-4 scene (1 M triangles, 128^3 grid), one window: the elide and trace legs of the default kernel and of the
+    grid_queue / grid_async kernels (which honour the elision too) give the same bits; elide traces fewer rays"""
+    import gen_mesh
+    tris = gen_mesh.soup(1 << 20)
+    lo, hi = gen_mesh.bbox_like_reference(tris)
+    sph = np.array([1024, 0, 0, 0, 145, 0, 0, 2048, 0], np.int32)
+    sq = np.array([4096, 0, 0, 0, 0, 0, 129, 0, 8192], np.int32)
+    lights = np.array([[10, 4, 10, 400], [15, 2, 7, 300]], np.float32)
+    with pt.Renderer(device=0) as r:
+        r.set_scene(pt.Scene(sph, sq, tris, lights, lo, hi))
+        r.build_grid(pt.grid_dims(r._scene))
+        W, H, spp, rows = 1920, 1080, 64, (540, 548)
+        tr = r.render("grid", W, H, SEED_SETS[0], rows=rows, spp=spp, want_accum=True, want_rng=True, dead_rays="trace")
+        for kernel in ("auto", "grid_queue", "grid_async"):
+            el = r.render("grid", W, H, SEED_SETS[0], rows=rows, spp=spp, kernel=kernel, want_accum=True, want_rng=True, dead_rays="elide")
+            r0, r1 = rows
+            assert np.array_equal(el.accum[r0:r1].view(np.uint32), tr.accum[r0:r1].view(np.uint32)), kernel
+            assert np.array_equal(el.rng_state.reshape(H, W, 4)[r0:r1], tr.rng_state.reshape(H, W, 4)[r0:r1]), kernel
+            assert np.array_equal(el.image[r0:r1], tr.image[r0:r1]), kernel
+            assert el.counters["samples"] == tr.counters["samples"], kernel
+            assert el.counters["rays"] < tr.counters["rays"], kernel
 
 
 @pytest.mark.parametrize("variant,dirname", [("base", "CLSuperPathTracer"), ("grid", "CLSuperPathTracer_trianglegrid")])

@@ -52,6 +52,48 @@ def test_trace_ray_golden(oracle_sep, scene_dirs):
     assert len(set(g["m_lmem"].tolist())) == 4    # the vectors cover sky, floor, diffuse and triangle hits
 
 
+def test_batched_trace_rays_equal_single_ray_probe(oracle_sep, scene_dirs):
+    """oracle_trace_rays (the batch entry the device probe is compared with) gives the golden rays the bits of
+    oracle_trace_ray (the entry the reference's own answers pin above)"""
+    g = np.load(os.path.join(G, "golden_trace.npz"))
+    sc = oracle_sep.load_scene_dir(scene_dirs["lmem"], "lmem")
+    for variant, carry in (("base", 0), ("lmem", 1)):
+        out = oracle_sep.trace_rays(variant, g["origins"], g["dirs"], g["t_in"], sc)
+        for k in range(0, g["origins"].shape[0], 7):
+            m, t, nn = oracle_sep.trace_ray(carry, g["origins"][k], g["dirs"][k], float(g["t_in"][k]), sc["spheres"], sc["squares"], sc["triangles"])
+            assert out["m"][k] == m and out["t"][k].view(np.uint32) == np.float32(t).view(np.uint32), (variant, k)
+            assert np.array_equal(out["n"][k].view(np.uint32), nn.view(np.uint32)), (variant, k)
+        assert np.array_equal(out["m"], g["m_" + variant]) and np.array_equal(out["t"].view(np.uint32), g["t_" + variant])
+        assert (out["cells"] == 0).all() and (out["tests"] == sc["triangles"].shape[0]).all()
+
+
+@pytest.mark.parametrize("oracle_name", ["oracle_sep", "oracle_fma"])
+def test_one_cell_grid_walk_equals_brute_force(request, scene_dirs, oracle_name):
+    """A 1x1x1 grid over a mesh of at most 62 triangles lists every triangle, in index order, in its one cell, and the
+    slab test has no lower bound on t: every ray whose line crosses the box tests all of them, as the brute-force scan
+    does.  So the grid walk and the scan must give the same material, t and normal bits, from inside and outside the box."""
+    o_lib = request.getfixturevalue(oracle_name)
+    sc = o_lib.load_scene_dir(scene_dirs["torus"], "grid")
+    assert sc["triangles"].shape[0] <= 62
+    lo, hi = sc["box_min"][:3].astype(np.float64), sc["box_max"][:3].astype(np.float64)
+    grid = {"box_min": sc["box_min"], "box_max": sc["box_max"], "res": np.array([1, 1, 1, 0], np.int32),
+            "cell_size": np.append((hi - lo), 0).astype(np.float32)}
+    rng = np.random.default_rng(3)
+    n = 40000
+    target = rng.uniform(lo, hi, (n, 3))
+    d = rng.normal(size=(n, 3))
+    d /= np.linalg.norm(d, axis=1, keepdims=True)
+    o = (target - rng.uniform(-3, 20, (n, 1)) * d).astype(np.float32)
+    d = rng.choice([-1.0, 1.0], (n, 1)) * (target - o)
+    d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(np.float32)
+    tin = np.full(n, 1e9, np.float32)
+    g = o_lib.trace_rays("grid", o, d, tin, sc, grid=grid)
+    b = o_lib.trace_rays("lmem", o, d, tin, sc)
+    assert np.array_equal(g["m"], b["m"]) and np.array_equal(g["t"].view(np.uint32), b["t"].view(np.uint32))
+    assert np.array_equal(g["n"].view(np.uint32), b["n"].view(np.uint32))
+    assert (g["m"] == 4).sum() > n // 10 and (g["t"] < 0).sum() > 0 and (g["cells"] == 1).mean() > 0.99
+
+
 @pytest.mark.parametrize("variant", ["base", "lmem", "nodof", "grid"])
 def test_image_rows_golden(oracle_sep, scene_dirs, variant):
     g = np.load(os.path.join(G, "golden_images.npz"))
