@@ -117,6 +117,8 @@ PTCUDA_SYMBOLS = {
     "pt_read_grid_cells": (_I, [_VP, _VP, C.c_size_t]),
     "pt_read_grid_csr": (_I, [_VP, _U32P, _U32P, C.POINTER(C.c_uint64)]),
     "pt_launch_pathtracer": (_VP, [_VP, C.POINTER(pt_camera), C.POINTER(pt_render_params)]),
+    "pt_launch_pathtracer_range": (_VP, [_VP, C.POINTER(pt_camera), C.POINTER(pt_render_params), _I, _I]),
+    "pt_set_render_state": (_I, [_VP, C.POINTER(pt_camera), C.POINTER(pt_render_params), _I, _FP, _U32P]),
     "pt_map_render": (_VP, [_VP, C.POINTER(_VP)]),
     "pt_read_accum": (_I, [_VP, _FP, C.c_size_t]),
     "pt_read_rng_state": (_I, [_VP, _U32P, C.c_size_t]),

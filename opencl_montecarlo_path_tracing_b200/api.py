@@ -344,11 +344,27 @@ class Renderer:
         _check(self._l.pt_read_vlp_grid_cells(self.ctx, raw.ctypes.data_as(C.c_void_p), ncells), "pt_read_vlp_grid_cells")
         return raw.reshape(ncells, 128)
 
-    def render(self, variant, width, height, seeds, read_image=True, **kw):
+    def render(self, variant, width, height, seeds, read_image=True, samples=None, **kw):
+        """Renders the frame in one launch, or with samples=(b, e) samples [b, e) of it as one range of a progression
+        (include/ptcuda.h, "progressive rendering"): the last range gives the one-launch frame bit for bit, earlier ones a
+        preview image.  accum / rng_state are read back when want_accum / want_rng are set.
+
+            kw = dict(spp=256)
+            for b, e in ((0, 16), (16, 64), (64, 256)):
+                out = r.render("base", 1920, 1080, seeds, samples=(b, e), **kw)      # out.image: preview, then the frame
+            # checkpoint after a range, and resume it later, in this or another Renderer with the same scene:
+            cp = r.render("base", 1920, 1080, seeds, samples=(0, 16), want_accum=True, want_rng=True, **kw)
+            r2.set_render_state("base", 1920, 1080, seeds, 16, cp.accum, cp.rng_state, **kw)
+            out = r2.render("base", 1920, 1080, seeds, samples=(16, 256), **kw)
+        """
         p = make_params(variant, width, height, seeds, **kw)
-        evt = self._l.pt_launch_pathtracer(self.ctx, C.byref(self.cam), C.byref(p))
+        if samples is None:
+            evt = self._l.pt_launch_pathtracer(self.ctx, C.byref(self.cam), C.byref(p))
+        else:
+            evt = self._l.pt_launch_pathtracer_range(self.ctx, C.byref(self.cam), C.byref(p), int(samples[0]), int(samples[1]))
         if not evt:
-            raise PtError("pt_launch_pathtracer failed: %s" % self._l.pt_last_error().decode())
+            raise PtError("%s failed: %s" % ("pt_launch_pathtracer" if samples is None else "pt_launch_pathtracer_range",
+                                             self._l.pt_last_error().decode()))
         image = None
         if read_image:
             ptr = self._l.pt_map_render(self.ctx, None)
@@ -370,6 +386,19 @@ class Renderer:
             _check(self._l.pt_read_rng_state(self.ctx, st.ctypes.data_as(C.POINTER(C.c_uint32)), st.size), "pt_read_rng_state")
             res.rng_state = st
         return res
+
+    def set_render_state(self, variant, width, height, seeds, samples_done, accum, rng_state, **kw):
+        """Restores a progression saved after samples_done samples (accum (H, W, 4) float32 and rng_state (H*W, 4) uint32, as
+        render(..., samples=(b, samples_done), want_accum=True, want_rng=True) returned them); keywords as for render().  The
+        next render(..., samples=(samples_done, e)) with the same params continues it."""
+        p = make_params(variant, width, height, seeds, **kw)
+        acc = np.ascontiguousarray(accum, np.float32)
+        st = np.ascontiguousarray(rng_state, np.uint32)
+        if acc.size != width * height * 4 or st.size != width * height * 4:
+            raise ValueError("set_render_state: accum and rng_state must hold width * height * 4 values each")
+        _check(self._l.pt_set_render_state(self.ctx, C.byref(self.cam), C.byref(p), int(samples_done),
+                                           acc.ctypes.data_as(C.POINTER(C.c_float)), st.ctypes.data_as(C.POINTER(C.c_uint32))),
+               "pt_set_render_state")
 
     def render_device(self, variant, width, height, seeds, d_rgba8, d_accum=None, **kw):
         """Render into caller-owned device memory (raw pointers, e.g. torch tensors' data_ptr())."""

@@ -11,8 +11,8 @@ namespace pt {
 struct LaunchArgs {
     Camera cam;
     uint4 seeds;
-    int W, H, spp;
-    float scale;            // 224/spp (3.5 at 64 spp)
+    int W, H, spp;          // spp: samples per pixel THIS launch runs (a range of a progression: its length)
+    float scale;            // 224/spp (3.5 at 64 spp) of the whole frame
     float c0, alpha;        // accumulation start value and alpha written to the float buffer: 13 / 255, or 0 / 0 for the
                             //   sample blocks b > 0 of a sample-sharded frame (pt_render_params.sample_blocks)
     int row_begin, row_end; // image rows [row_begin, row_end) are eligible
@@ -37,6 +37,12 @@ struct LaunchArgs {
     const uint32_t *vg_start, *vg_refs;
     float vg_bmin[3], vg_cell[3];
     int vg_res[3];
+    // progressive rendering (pt_launch_pathtracer_range): a range that does not start at sample 0 continues every pixel from
+    // the colour sum and RNG state the previous range left (NULL: seed from `seeds`, start at c0); a range that does not end
+    // the frame writes the preview ((c - 13) * preview) + 13 into rgba, preview = spp / end (0: the colour itself)
+    const float4 *accum_in;
+    const uint4 *rng_in;
+    float preview;
 };
 
 // virtual row -> image row (identity, or the rank's interleaved stripes)
@@ -51,6 +57,14 @@ __host__ __device__ inline int map_row(const LaunchArgs &P, int vr) {
 struct pt_event_s {
     cudaEvent_t start, stop;
     int device;
+};
+
+// What has to stay the same over the ranges of one progression (memcmp'ed: built from a zeroed object)
+struct pt_progression_key {
+    int variant, width, height, spp, arith, row_begin, row_end, row_interleave, rank, nranks;
+    uint32_t seeds[4];
+    pt_camera cam;
+    uint64_t scene_version, grid_version, vpl_version, vlp_grid_version;   // the inputs the variant reads (0: not read)
 };
 
 struct pt_ctx_s {
@@ -107,6 +121,12 @@ struct pt_ctx_s {
     int last_kernel;              // PT_KERNEL_* the most recent render resolved to (after PT_KERNEL_AUTO)
     int accum_valid_w, accum_valid_h;   // extent of d_accum the most recent launch wrote (0: it did not request it)
     size_t rng_valid_items;             // work-items of d_rng the most recent launch wrote
+
+    // progressive rendering: d_accum / d_rng hold the state of this progression after its first `prog_next` samples
+    bool prog_active;
+    int prog_next;
+    pt_progression_key prog_key;
+    uint64_t grid_version, vpl_version, vlp_grid_version;   // bumped by every grid build, VPL buffer change, VLP grid build
 
     // bidirectional variant: VPL buffer as the reference defines it + its compacted non-zero entries
     bool vpls_set;

@@ -87,6 +87,36 @@ PT_DEV void flush_counters(const LaunchArgs &P, const Counters &c, int ntri_coun
     }
 }
 
+// The state a pixel's sample loop carries from one sample to the next is its colour sum and its RNG state, nothing else.
+// A launch starts it fresh (seeded from the pixel id, the bias c0) or, continuing a progression, where the previous
+// range of it left the pixel.  Read once, before the sample loop.
+PT_DEV void pixel_state_in(const LaunchArgs &P, uint32_t pix, Rng &rng, float &cx, float &cy, float &cz) {
+    if (P.rng_in) {
+        const uint4 r = P.rng_in[pix];
+        const float4 a = P.accum_in[pix];
+        rng.x0 = r.x; rng.x1 = r.y; rng.c0 = r.z; rng.c1 = r.w;
+        cx = a.x; cy = a.y; cz = a.z;
+    } else {
+        rng = rng_seed(P.seeds, pix);
+        cx = cy = cz = P.c0;
+    }
+}
+
+// convert_uchar4 of the colour sum (or, on a range that does not end the frame, of the preview ((c - 13) * f) + 13 with
+// f = spp / samples done, each operation rounded on its own), plus the optional float buffer and final RNG state.  The
+// thread that read the pixel's state writes it, so input and output of a range may be the same buffers.
+PT_DEV void pixel_state_out(const LaunchArgs &P, size_t pix, const Rng &rng, float cx, float cy, float cz) {
+    if (P.preview != 0.0f) {
+        const float f = P.preview;
+        P.rgba[pix] = pack_rgba8_rz(__fadd_rn(__fmul_rn(__fsub_rn(cx, 13.0f), f), 13.0f), __fadd_rn(__fmul_rn(__fsub_rn(cy, 13.0f), f), 13.0f),
+                                    __fadd_rn(__fmul_rn(__fsub_rn(cz, 13.0f), f), 13.0f), P.alpha);
+    } else {
+        P.rgba[pix] = pack_rgba8_rz(cx, cy, cz, P.alpha);
+    }
+    if (P.accum) P.accum[pix] = make_float4(cx, cy, cz, P.alpha);
+    if (P.rng_out) P.rng_out[pix] = make_uint4(rng.x0, rng.x1, rng.c0, rng.c1);
+}
+
 // BIG, trianglegrid: grids whose records do not stay in L1 — 64 registers / 8 CTAs per SM (72 / 7: 14.78 vs 14.51 ms per 16 spp)
 // and the longest-tile-first launch order; otherwise 80 registers / 6 CTAs.  Both use the single ray loop (PT_BIG_TWO_TRACES).
 // BIG, brute-force variants: frames above 400 k pixels — per-cluster triangle culling compiled in (tri_loop<.., CL>).
@@ -116,8 +146,9 @@ __global__ void __launch_bounds__(128, (BIG && VARIANT == PT_VARIANT_GRID) ? 8 :
     Counters cnt = {0, 0, 0, 0, 0, 0};
     const int j = map_row(P, vr);
     if (i < P.W && vr < P.nrows && j < P.row_end) {
-        Rng rng = rng_seed(P.seeds, (uint32_t)(j * P.W + i));
-        float cx = P.c0, cy = P.c0, cz = P.c0;
+        Rng rng;
+        float cx, cy, cz;
+        pixel_state_in(P, (uint32_t)(j * P.W + i), rng, cx, cy, cz);
         for (int s = 0; s < P.spp; ++s) {
             V3 o, d;
             camera_ray<FMA>(P.cam, rng, i, j, o, d);
@@ -127,10 +158,7 @@ __global__ void __launch_bounds__(128, (BIG && VARIANT == PT_VARIANT_GRID) ? 8 :
             cy = Ar<FMA>::madd(c.y, P.scale, cy);
             cz = Ar<FMA>::madd(c.z, P.scale, cz);
         }
-        const size_t pix = (size_t)j * P.W + i;
-        P.rgba[pix] = pack_rgba8_rz(cx, cy, cz, P.alpha);
-        if (P.accum) P.accum[pix] = make_float4(cx, cy, cz, P.alpha);
-        if (P.rng_out) P.rng_out[pix] = make_uint4(rng.x0, rng.x1, rng.c0, rng.c1);
+        pixel_state_out(P, (size_t)j * P.W + i, rng, cx, cy, cz);
     }
     if (GRID) cnt.btests = cnt.gtri;        // trace_grid tests every record of the cells it visits
     flush_counters(P, cnt, GRID ? 0 : S->ntri_counted, P.ap.nsq + P.ap.nsp);
@@ -199,7 +227,9 @@ __global__ void __launch_bounds__(256, 4) k_mega_nodof(const __grid_constant__ L
 // scene with the same geometry is merely a worse order.  (Tried and dropped: classifying tiles by "primary ray hits the
 // grid box" — no gain, floor tiles are as expensive, their shadow rays cross the grid; a 1-spp pre-pass as the cost
 // estimate for the FIRST launch — its order was no better than raster, one sample per pixel says too little about 256;
-// 1-warp CTAs, to shrink the unit — 3 % slower.)
+// 1-warp CTAs, to shrink the unit — 3 % slower.)  The key is the geometry, not the sample count: a progression in ranges
+// of >= 16 samples (pt_launch_pathtracer_range) records in its first range and runs sorted from its second on, and a
+// one-launch frame after it on the same context reuses that order.
 struct TileOrderKey {
     int W, H, row_begin, row_end, nrows, stripe_h, rank, nranks, variant_fma, ntri;
     unsigned long long scene_version;

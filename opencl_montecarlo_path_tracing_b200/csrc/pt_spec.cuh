@@ -26,7 +26,7 @@
 namespace pt {
 
 struct SpecEntry {            // 48 bytes
-    uint32_t pix, sdone;      // linear pixel index, samples already accumulated
+    uint32_t pix, sdone;      // linear pixel index, samples of THIS launch already accumulated (P.spp = the launch's samples)
     float cx, cy;
     float cz, pad0, pad1, pad2;
     uint4 rng;                // state at the start of sample `sdone`
@@ -48,7 +48,7 @@ __global__ void __launch_bounds__(128, 7) k_spec_light(const __grid_constant__ L
     float cx = P.c0, cy = P.c0, cz = P.c0;
     int s = 0;
     const bool mine = i < P.W && vr < P.nrows && j < P.row_end;
-    if (mine) rng = rng_seed(P.seeds, (uint32_t)(j * P.W + i));
+    if (mine) pixel_state_in(P, (uint32_t)(j * P.W + i), rng, cx, cy, cz);
     // Every lane of the warp walks this loop together and re-converges once per sample.  (Written as a per-lane loop with a
     // `break` for the lanes that leave, the base variant's warps never re-converged after their first divergent sample: one
     // 8x4 tile on a sphere's terminator ran its 32 lanes one after the other — 6.9 M cycles, 3.7 ms for the whole pass.)
@@ -75,12 +75,7 @@ __global__ void __launch_bounds__(128, 7) k_spec_light(const __grid_constant__ L
         __syncwarp();
         if (!__any_sync(0xffffffffu, live)) break;
     }
-    if (mine && !queued) {
-        const size_t pix = (size_t)j * P.W + i;
-        P.rgba[pix] = pack_rgba8_rz(cx, cy, cz, P.alpha);
-        if (P.accum) P.accum[pix] = make_float4(cx, cy, cz, P.alpha);
-        if (P.rng_out) P.rng_out[pix] = make_uint4(rng.x0, rng.x1, rng.c0, rng.c1);
-    }
+    if (mine && !queued) pixel_state_out(P, (size_t)j * P.W + i, rng, cx, cy, cz);
     // one warp-aggregated atomicAdd reserves the queue slots of the warp's heavy pixels
     const unsigned qm = __ballot_sync(0xffffffffu, queued);
     if (qm) {
@@ -259,11 +254,7 @@ __global__ void __launch_bounds__(128, 6) k_spec_heavy(const __grid_constant__ L
             base.c0 = __shfl_sync(0xffffffffu, r.c0, lastv); base.c1 = __shfl_sync(0xffffffffu, r.c1, lastv);
             k0 += __popc(valid);
         }
-        if (lane == 0) {
-            P.rgba[E.pix] = pack_rgba8_rz(cx, cy, cz, P.alpha);
-            if (P.accum) P.accum[E.pix] = make_float4(cx, cy, cz, P.alpha);
-            if (P.rng_out) P.rng_out[E.pix] = make_uint4(base.x0, base.x1, base.c0, base.c1);
-        }
+        if (lane == 0) pixel_state_out(P, E.pix, base, cx, cy, cz);
     }
     flush_counters(P, cnt, S->ntri_counted, P.ap.nsq + P.ap.nsp);
 }

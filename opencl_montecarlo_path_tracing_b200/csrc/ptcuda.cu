@@ -440,6 +440,7 @@ extern "C" pt_event pt_build_grid(pt_ctx c, const pt_grid *g) {
     PT_CUDA_NULL(cudaSetDevice(c->device), "select device");
     pt_event e = event_new(c);
     if (!e) return nullptr;
+    c->grid_version++;
     cudaEventRecord(e->start, c->stream);
     if (pt_grid_build_device(c, g)) { pt_release_event(e); return nullptr; }
     cudaEventRecord(e->stop, c->stream);
@@ -501,6 +502,7 @@ extern "C" pt_event pt_build_vlp_grid(pt_ctx c, const pt_grid *g) {
     PT_CUDA_NULL(cudaSetDevice(c->device), "select device");
     pt_event e = event_new(c);
     if (!e) return nullptr;
+    c->vlp_grid_version++;
     cudaEventRecord(e->start, c->stream);
     if (pt_vlp_grid_build_device(c, g)) { pt_release_event(e); return nullptr; }
     cudaEventRecord(e->stop, c->stream);
@@ -759,9 +761,8 @@ static pt_render_params resolve_auto(pt_ctx c, const pt_render_params *in, const
     return p;
 }
 
-static int dispatch(pt_ctx c, const pt_render_params *pin, const pt::LaunchArgs &A) {
-    const pt_render_params resolved = resolve_auto(c, pin, A);
-    const pt_render_params *p = &resolved;
+// p: the params as resolve_auto left them
+static int dispatch(pt_ctx c, const pt_render_params *p, const pt::LaunchArgs &A) {
     c->last_kernel = p->kernel;
     DevLock lock(c->device);     // constant-scene bind + launch are one critical section per device
     PT_CUDA(cudaMemsetAsync(c->d_counters, 0, 8 * sizeof(unsigned long long), c->stream), "clear counters");
@@ -792,33 +793,113 @@ static int dispatch(pt_ctx c, const pt_render_params *pin, const pt::LaunchArgs 
     return pt_fail(1, "render: unknown kernel kind %d", p->kernel);
 }
 
-extern "C" pt_event pt_launch_pathtracer(pt_ctx c, const pt_camera *cam, const pt_render_params *p) {
-    if (!c || !cam || !p) { pt_fail(1, "pt_launch_pathtracer: null argument"); return nullptr; }
+// ---- progressive rendering: checks shared by range launches and pt_set_render_state, and the progression key
+static int progression_params(pt_ctx c, const pt_camera *cam, const pt_render_params *p, const char *who, pt_progression_key *key) {
+    if (p->variant == PT_VARIANT_NODOF)
+        return pt_fail(1, "%s: the NoDoF variant has no per-pixel sample chain to continue (64 streams per pixel, fixed 8x8 reduction)", who);
+    if (p->sample_blocks > 1) return pt_fail(1, "%s: sample_blocks > 1 (sample sharding) cannot be rendered in ranges", who);
+    memset(key, 0, sizeof(*key));
+    key->variant = p->variant; key->width = p->width; key->height = p->height; key->spp = p->spp;
+    key->arith = p->arith != PT_ARITH_SEPARATE ? PT_ARITH_FMA : PT_ARITH_SEPARATE;
+    key->row_begin = p->row_begin; key->row_end = p->row_end;
+    key->row_interleave = p->row_interleave; key->rank = p->rank; key->nranks = p->nranks;
+    memcpy(key->seeds, p->seeds, sizeof(key->seeds));
+    key->cam = *cam;
+    key->scene_version = c->scene_version;
+    if (p->variant == PT_VARIANT_GRID) key->grid_version = c->grid_version;
+    if (p->variant == PT_VARIANT_BIDIR || p->variant == PT_VARIANT_VLPGRID) key->vpl_version = c->vpl_version;
+    if (p->variant == PT_VARIANT_VLPGRID) key->vlp_grid_version = c->vlp_grid_version;
+    return 0;
+}
+
+// The one-launch render (range == false: samples [0, spp), state kept only as want_accum / want_rng ask) and a range
+// [b, e) of a progression (state always kept in d_accum / d_rng) share validation, fill_args and dispatch.
+static pt_event launch_render(pt_ctx c, const pt_camera *cam, const pt_render_params *p, bool range, int b, int e) {
+    const char *who = range ? "pt_launch_pathtracer_range" : "pt_launch_pathtracer";
+    if (!c || !cam || !p) { pt_fail(1, "%s: null argument", who); return nullptr; }
     if (validate_params(c, p)) return nullptr;
+    pt_progression_key key;
+    if (range) {
+        if (progression_params(c, cam, p, who, &key)) return nullptr;
+        if (b < 0 || e <= b || e > p->spp) { pt_fail(1, "%s: samples [%d, %d) are not a range of [0, %d)", who, b, e, p->spp); return nullptr; }
+        if (b > 0) {
+            if (!c->prog_active) { pt_fail(1, "%s: sample %d continues no progression (start at 0 or pt_set_render_state)", who, b); return nullptr; }
+            if (memcmp(&key, &c->prog_key, sizeof(key)) != 0) {
+                pt_fail(1, "%s: params, camera, scene, grid or VPLs differ from the progression's", who);
+                return nullptr;
+            }
+            if (b != c->prog_next) { pt_fail(1, "%s: the progression continues at sample %d, not %d", who, c->prog_next, b); return nullptr; }
+        }
+    }
     PT_CUDA_NULL(cudaSetDevice(c->device), "select device");
     const size_t npix = (size_t)p->width * p->height;
     const size_t nitems = p->variant == PT_VARIANT_NODOF ? npix * 64 : npix;
+    const bool keep_accum = range || p->want_accum, keep_rng = range || p->want_rng;
+    // (a continuation has the key of the range before it, so the same size: these never grow, never lose the state)
     if (ensure_dev((void **)&c->d_rgba, &c->rgba_cap, npix * 4)) return nullptr;
-    if (p->want_accum && ensure_dev((void **)&c->d_accum, &c->accum_cap, npix * 16)) return nullptr;
-    if (p->want_rng && ensure_dev((void **)&c->d_rng, &c->rng_cap, nitems * 16)) return nullptr;
+    if (keep_accum && ensure_dev((void **)&c->d_accum, &c->accum_cap, npix * 16)) return nullptr;
+    if (keep_rng && ensure_dev((void **)&c->d_rng, &c->rng_cap, nitems * 16)) return nullptr;
     pt::LaunchArgs A;
-    fill_args(c, cam, p, c->d_rgba, p->want_accum ? c->d_accum : nullptr, p->want_rng ? c->d_rng : nullptr, &A);
+    fill_args(c, cam, p, c->d_rgba, keep_accum ? c->d_accum : nullptr, keep_rng ? c->d_rng : nullptr, &A);
+    if (range) {
+        A.spp = e - b;                                         // loop count; A.scale stays 224 / spp of the frame
+        if (b > 0) { A.accum_in = c->d_accum; A.rng_in = c->d_rng; }
+        if (e < p->spp) A.preview = (float)p->spp / (float)e;
+    }
+    const pt_render_params resolved = resolve_auto(c, p, A);
+    if (range && resolved.kernel != PT_KERNEL_MEGA && resolved.kernel != PT_KERNEL_SPEC) {
+        pt_fail(1, "%s: kernel flavour %d cannot render sample ranges; MEGA, SPEC and AUTO can", who, resolved.kernel);
+        return nullptr;
+    }
+    c->prog_active = false;                 // from here on the state buffers may be overwritten
     const bool partial = A.nrows != p->height || A.stripe_h > 0;
     if (partial) {
         cudaMemsetAsync(c->d_rgba, 0, npix * 4, c->stream);
-        if (p->want_accum) cudaMemsetAsync(c->d_accum, 0, npix * 16, c->stream);
-        if (p->want_rng) cudaMemsetAsync(c->d_rng, 0, nitems * 16, c->stream);
+        if (keep_accum && b == 0) cudaMemsetAsync(c->d_accum, 0, npix * 16, c->stream);
+        if (keep_rng && b == 0) cudaMemsetAsync(c->d_rng, 0, nitems * 16, c->stream);
     }
-    pt_event e = event_new(c);
-    if (!e) return nullptr;
-    cudaEventRecord(e->start, c->stream);
-    if (dispatch(c, p, A)) { pt_release_event(e); return nullptr; }
-    cudaEventRecord(e->stop, c->stream);
+    pt_event ev = event_new(c);
+    if (!ev) return nullptr;
+    cudaEventRecord(ev->start, c->stream);
+    if (dispatch(c, &resolved, A)) { pt_release_event(ev); return nullptr; }
+    cudaEventRecord(ev->stop, c->stream);
     c->last_w = p->width; c->last_h = p->height; c->last_variant = p->variant;
     // what pt_read_accum / pt_read_rng_state may copy: only what THIS launch wrote
-    c->accum_valid_w = p->want_accum ? p->width : 0; c->accum_valid_h = p->want_accum ? p->height : 0;
-    c->rng_valid_items = p->want_rng ? nitems : 0;
-    return e;
+    c->accum_valid_w = keep_accum ? p->width : 0; c->accum_valid_h = keep_accum ? p->height : 0;
+    c->rng_valid_items = keep_rng ? nitems : 0;
+    if (range) { c->prog_active = true; c->prog_key = key; c->prog_next = e; }
+    return ev;
+}
+
+extern "C" pt_event pt_launch_pathtracer(pt_ctx c, const pt_camera *cam, const pt_render_params *p) {
+    return launch_render(c, cam, p, false, 0, p ? p->spp : 0);
+}
+
+extern "C" pt_event pt_launch_pathtracer_range(pt_ctx c, const pt_camera *cam, const pt_render_params *p, int sample_begin,
+                                               int sample_end) {
+    return launch_render(c, cam, p, true, sample_begin, sample_end);
+}
+
+extern "C" int pt_set_render_state(pt_ctx c, const pt_camera *cam, const pt_render_params *p, int samples_done, const float *accum,
+                                   const uint32_t *rng_state) {
+    const char *who = "pt_set_render_state";
+    if (!c || !cam || !p || !accum || !rng_state) return pt_fail(1, "%s: null argument", who);
+    int rc = validate_params(c, p);
+    if (rc) return rc;
+    pt_progression_key key;
+    rc = progression_params(c, cam, p, who, &key);
+    if (rc) return rc;
+    if (samples_done <= 0 || samples_done >= p->spp) return pt_fail(1, "%s: samples_done %d outside (0, %d)", who, samples_done, p->spp);
+    PT_CUDA(cudaSetDevice(c->device), "select device");
+    const size_t npix = (size_t)p->width * p->height;
+    c->prog_active = false;
+    if (ensure_dev((void **)&c->d_accum, &c->accum_cap, npix * 16) || ensure_dev((void **)&c->d_rng, &c->rng_cap, npix * 16)) return 1;
+    PT_CUDA(cudaMemcpyAsync(c->d_accum, accum, npix * 16, cudaMemcpyHostToDevice, c->stream), "upload accumulation buffer");
+    PT_CUDA(cudaMemcpyAsync(c->d_rng, rng_state, npix * 16, cudaMemcpyHostToDevice, c->stream), "upload RNG states");
+    PT_CUDA(cudaStreamSynchronize(c->stream), "sync state upload");     // the host buffers may be pageable
+    c->accum_valid_w = p->width; c->accum_valid_h = p->height; c->rng_valid_items = npix;
+    c->prog_active = true; c->prog_key = key; c->prog_next = samples_done;
+    return 0;
 }
 
 // ------------------------------------------------------------------------------- bidirectional: VPLs
@@ -853,6 +934,7 @@ extern "C" pt_event pt_launch_lighttracer(pt_ctx c, int n_vlp_per_light, const u
     fill_args(c, &cam0, &rp0, nullptr, nullptr, nullptr, &LA);
     pt_event e = event_new(c);
     if (!e) return nullptr;
+    c->vpl_version++;
     cudaEventRecord(e->start, c->stream);
     DevLock lock(c->device);
     if (pt_launch_light_tracer_kernels(c, ar, LA, n_vlp_per_light, c->d_vpls, nullptr, c->d_vpl_active, c->d_vpl_count)) {
@@ -898,6 +980,7 @@ extern "C" pt_event pt_launch_metropolis_lighttracer(pt_ctx c, int n_paths_per_l
     fill_args(c, &cam0, &rp0, nullptr, nullptr, nullptr, &LA);
     pt_event e = event_new(c);
     if (!e) return nullptr;
+    c->vpl_version++;
     cudaEventRecord(e->start, c->stream);
     DevLock lock(c->device);
     if (pt_launch_metropolis_kernels(c, ar, LA, n_paths_per_light, mutation_rounds, c->d_vpls, c->d_metro_seed, c->d_metro_mutated,
@@ -930,6 +1013,7 @@ extern "C" int pt_read_metropolis_paths(pt_ctx c, uint32_t *paths, int capacity_
 extern "C" int pt_set_vpls(pt_ctx c, const float *vpls, int n) {
     if (!c || n < 0 || (n > 0 && !vpls)) return pt_fail(1, "pt_set_vpls: bad argument");
     PT_CUDA(cudaSetDevice(c->device), "select device");
+    c->vpl_version++;
     int rc = ensure_vpls(c, n);
     if (rc) return rc;
     if (n > 0) PT_CUDA(cudaMemcpyAsync(c->d_vpls, vpls, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, c->stream), "upload VPLs");
@@ -963,7 +1047,9 @@ extern "C" int pt_render_device(pt_ctx c, const pt_camera *cam, const pt_render_
     pt::LaunchArgs A;
     fill_args(c, cam, p, (uint32_t *)d_rgba8, (float4 *)d_accum_f32, nullptr, &A);
     c->last_variant = p->variant;
-    return dispatch(c, p, A);
+    c->prog_active = false;
+    const pt_render_params resolved = resolve_auto(c, p, A);
+    return dispatch(c, &resolved, A);
 }
 
 extern "C" void *pt_map_render(pt_ctx c, pt_event *evt) {
