@@ -255,6 +255,36 @@ static void decode_bitmap(const int32_t bm[9], bool sphere, float2 *out, int *n)
     *n = c;
 }
 
+// Bounding sphere of triangles src[0..n) of `tris` (src == nullptr: triangles 0..n-1) for the conservative line/sphere
+// culls (pt_device.cuh, AnalyticParams::mesh_*): the centre of the vertices' box, rounded to float, and the largest distance
+// (double) from that FLOAT centre to a vertex, inflated by 1 % + 0.01 and rounded up to a float.  Measuring the radius from
+// the stored centre keeps every vertex inside however far the mesh lies from the origin (there half an ulp of the centre
+// outgrows the 0.01); the inflation covers the float rounding of the device's line/sphere test.  Non-finite radius: +inf.
+static float4 tri_bounding_sphere(const float *tris, const int *src, int n) {
+    double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
+    for (int k = 0; k < n; ++k)
+        for (int v = 0; v < 3; ++v)
+            for (int a = 0; a < 3; ++a) {
+                const double x = tris[12 * (size_t)(src ? src[k] : k) + 4 * v + a];
+                if (x < lo[a]) lo[a] = x;
+                if (x > hi[a]) hi[a] = x;
+            }
+    float ctr[3] = {0.f, 0.f, 0.f};
+    if (n > 0) for (int a = 0; a < 3; ++a) ctr[a] = (float)(0.5 * (lo[a] + hi[a]));
+    double r2 = 0;
+    for (int k = 0; k < n; ++k)
+        for (int v = 0; v < 3; ++v) {
+            const float *q = tris + 12 * (size_t)(src ? src[k] : k) + 4 * v;
+            const double dx = (double)q[0] - ctr[0], dy = (double)q[1] - ctr[1], dz = (double)q[2] - ctr[2];
+            const double d2 = dx * dx + dy * dy + dz * dz;
+            if (d2 > r2) r2 = d2;
+        }
+    const double r = sqrt(r2) * 1.01 + 0.01;
+    float rf = isfinite(r) ? (float)r : INFINITY;
+    if ((double)rf < r) rf = nextafterf(rf, INFINITY);
+    return make_float4(ctr[0], ctr[1], ctr[2], rf);
+}
+
 extern "C" int pt_set_scene(pt_ctx c, const pt_scene *sc) {
     using namespace pt;
     if (!c || !sc) return pt_fail(1, "pt_set_scene: null argument");
@@ -298,54 +328,17 @@ extern "C" int pt_set_scene(pt_ctx c, const pt_scene *sc) {
             ++kept;
         }
         S->ntri = kept;
-        // bounding sphere of every cluster of PT_CLUSTER consecutive records (double precision, radius inflated by
-        // 1 % + 0.01 exactly like the whole-mesh sphere below)
+        // bounding sphere of every cluster of PT_CLUSTER consecutive records, built like the whole-mesh sphere below
         S->ncl = (kept + PT_CLUSTER - 1) / PT_CLUSTER;
         for (int cl = 0; cl < S->ncl; ++cl) {
-            double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
             const int k0 = cl * PT_CLUSTER, k1 = k0 + PT_CLUSTER < kept ? k0 + PT_CLUSTER : kept;
-            for (int k = k0; k < k1; ++k)
-                for (int v = 0; v < 3; ++v)
-                    for (int ax = 0; ax < 3; ++ax) {
-                        double x = sc->triangles[12 * (size_t)kept_src[k] + 4 * v + ax];
-                        if (x < lo[ax]) lo[ax] = x;
-                        if (x > hi[ax]) hi[ax] = x;
-                    }
-            double ctr[3], r2 = 0;
-            for (int ax = 0; ax < 3; ++ax) ctr[ax] = 0.5 * (lo[ax] + hi[ax]);
-            for (int k = k0; k < k1; ++k)
-                for (int v = 0; v < 3; ++v) {
-                    const float *q = sc->triangles + 12 * (size_t)kept_src[k] + 4 * v;
-                    double dx = q[0] - ctr[0], dy = q[1] - ctr[1], dz = q[2] - ctr[2];
-                    double d2 = dx * dx + dy * dy + dz * dz;
-                    if (d2 > r2) r2 = d2;
-                }
-            double rr = sqrt(r2) * 1.01 + 0.01;
-            S->csph[cl] = make_float4((float)ctr[0], (float)ctr[1], (float)ctr[2], isfinite(rr) ? (float)rr : INFINITY);
+            S->csph[cl] = tri_bounding_sphere(sc->triangles, kept_src + k0, k1 - k0);
         }
     }
     c->scene_bytes = (int)(offsetof(SceneBlock, tri) + (size_t)kept * 48);
     {
-        // bounding sphere of the brute-force triangles' vertices (double precision), radius inflated by
-        // 1 % + 0.01 — far beyond any float rounding of the line/sphere test or of Moller-Trumbore
-        double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
-        for (int i = 0; i < nbrute; ++i)
-            for (int v = 0; v < 3; ++v)
-                for (int a = 0; a < 3; ++a) {
-                    double x = sc->triangles[12 * (size_t)i + 4 * v + a];
-                    if (x < lo[a]) lo[a] = x;
-                    if (x > hi[a]) hi[a] = x;
-                }
-        double ctr[3] = {0, 0, 0}, r2 = 0;
-        if (nbrute > 0) for (int a = 0; a < 3; ++a) ctr[a] = 0.5 * (lo[a] + hi[a]);
-        for (int i = 0; i < nbrute; ++i)
-            for (int v = 0; v < 3; ++v) {
-                double dx = sc->triangles[12 * (size_t)i + 4 * v] - ctr[0], dy = sc->triangles[12 * (size_t)i + 4 * v + 1] - ctr[1],
-                       dz = sc->triangles[12 * (size_t)i + 4 * v + 2] - ctr[2];
-                double q = dx * dx + dy * dy + dz * dz;
-                if (q > r2) r2 = q;
-            }
-        double r = sqrt(r2) * 1.01 + 0.01;
+        // bounding sphere of the brute-force triangles' vertices
+        const float4 sph = tri_bounding_sphere(sc->triangles, nullptr, nbrute);
         double kmax = 0;     // max |e0||e2| over the brute-force triangles
         for (int i = 0; i < nbrute; ++i) {
             const float *t = sc->triangles + 12 * (size_t)i;
@@ -353,8 +346,8 @@ extern "C" int pt_set_scene(pt_ctx c, const pt_scene *sc) {
             double e2 = sqrt(pow((double)t[8] - t[0], 2) + pow((double)t[9] - t[1], 2) + pow((double)t[10] - t[2], 2));
             if (e0 * e2 > kmax) kmax = e0 * e2;
         }
-        for (int a = 0; a < 3; ++a) c->mesh_c[a] = (float)ctr[a];
-        c->mesh_r = (float)r;
+        c->mesh_c[0] = sph.x; c->mesh_c[1] = sph.y; c->mesh_c[2] = sph.z;
+        c->mesh_r = sph.w;
         c->mesh_k = (float)(2e-4 * kmax + 1e-6);
         if (!isfinite(c->mesh_r) || !isfinite(c->mesh_k)) c->mesh_r = INFINITY;
     }
