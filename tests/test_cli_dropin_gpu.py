@@ -2,6 +2,7 @@
 result.ppm whose bytes equal what the oracle writes for the printed seeds."""
 import os
 import re
+import shutil
 import subprocess
 
 import numpy as np
@@ -49,6 +50,28 @@ def test_cli_matches_oracle(scene_dirs, oracle_fma, variant, args):
     oracle_fma.save_pam(tmp, ref["image"])
     assert open(os.path.join(d, "result.ppm"), "rb").read() == open(tmp, "rb").read()
     assert ("Processing image %dx%d with data size %d bytes" % (w, h, w * h * 4)) in out
+
+
+@pytest.mark.parametrize("variant", ["base", "lmem"])
+@pytest.mark.parametrize("nlights", [1, 5])
+def test_cli_other_light_counts(scene_dirs, oracle_fma, tmp_path, variant, nlights):
+    """The executables' default 512x512 frame (AUTO picks the speculative kernel there) with a lights.txt of 1 and 5 lights"""
+    from test_spec_kernel_gpu import FIVE_LIGHTS
+    d = str(tmp_path / variant)
+    shutil.copytree(scene_dirs[variant], d)
+    with open(os.path.join(d, "lights.txt"), "w") as f:
+        f.write("\n".join("%g" % v for v in FIVE_LIGHTS[:nlights].reshape(-1)))
+    exe = os.path.join(BIN, DIRS[variant], "CLSuperPathTracer")
+    env = dict(os.environ, PT_SEEDS="123456789,42,7,99999")
+    p = subprocess.run([exe], cwd=d, env=env, capture_output=True, text=True, timeout=300)
+    assert p.returncode == 0, p.stderr
+    assert ("Number of lights: %d" % nlights) in p.stdout and "Processing image 512x512" in p.stdout
+    osc = oracle_fma.load_scene_dir(d, variant)
+    assert np.array_equal(osc["lights"], FIVE_LIGHTS[:nlights])
+    ref = oracle_fma.render(variant, 512, 512, (123456789, 42, 7, 99999), osc, want_accum=False, want_rng=False)
+    tmp = os.path.join(d, "oracle_expected.ppm")
+    oracle_fma.save_pam(tmp, ref["image"])
+    assert open(os.path.join(d, "result.ppm"), "rb").read() == open(tmp, "rb").read()
 
 
 def test_cli_wall_clock_seeds_and_error_convention(scene_dirs, tmp_path):

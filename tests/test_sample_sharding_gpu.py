@@ -6,6 +6,7 @@ import pytest
 
 import opencl_montecarlo_path_tracing_b200 as pt
 from conftest import SEED_SETS
+from test_spec_kernel_gpu import FIVE_LIGHTS
 
 pytestmark = pytest.mark.gpu
 W = H = 512
@@ -25,8 +26,9 @@ def _setup(renderer, scene_dirs, o, variant):
     return o.load_scene_dir(d, variant), extra
 
 
-@pytest.mark.parametrize("variant,kernels", [("base", ("mega", "persistent", "wavefront")), ("lmem", ("mega", "persistent")),
-                                             ("grid", ("mega", "persistent", "wavefront", "grid_tma", "grid_stream", "grid_pool")),
+@pytest.mark.parametrize("variant,kernels", [("base", ("mega", "persistent", "wavefront", "spec")), ("lmem", ("mega", "persistent", "spec")),
+                                             ("grid", ("mega", "persistent", "wavefront", "grid_tma", "grid_stream", "grid_pool", "grid_queue",
+                                                       "grid_async")),
                                              ("bidir", ("mega",))])
 def test_blocks_bit_exact_and_sum_to_the_frame(renderer, scene_dirs, oracle_fma, variant, kernels):
     osc, extra = _setup(renderer, scene_dirs, oracle_fma, variant)
@@ -53,6 +55,34 @@ def test_blocks_bit_exact_and_sum_to_the_frame(renderer, scene_dirs, oracle_fma,
     b0 = renderer.render(variant, W, H, SEED_SETS[0], rows=ROWS, sample_block=0, sample_blocks=R, want_rng=True)
     short = oracle_fma.render(variant, W, H, SEED_SETS[0], osc, rows=ROWS, spp=16, **extra)
     assert np.array_equal(b0.rng_state.reshape(H, W, 4)[r0:r1], short["rng_state"].reshape(H, W, 4)[r0:r1])
+
+
+@pytest.mark.parametrize("nlights", [1, 5])
+def test_blocks_at_other_light_counts(renderer, scene_dirs, oracle_fma, nlights):
+    """Blocks b > 0 (own seeds, no bias 13) with an odd light count: a hit sample draws 2 + nlights pairs"""
+    lights = FIVE_LIGHTS[:nlights]
+    R = 4
+    r0, r1 = ROWS
+    for variant, kernels in (("base", ("mega", "spec")), ("lmem", ("spec", "wavefront")), ("grid", ("mega", "grid_queue", "grid_async"))):
+        d = scene_dirs[variant]
+        scene = pt.load_scene_dir(d, variant)
+        scene.lights = lights
+        renderer.set_scene(scene)
+        if variant == "grid":
+            renderer.build_grid(pt.grid_dims(scene))
+        osc = oracle_fma.load_scene_dir(d, variant)
+        osc["lights"] = lights
+        for b in range(R):
+            ref = oracle_fma.render(variant, W, H, SEED_SETS[0], osc, rows=ROWS, sample_block=b, sample_blocks=R)
+            assert ref["counters"]["shadow_rays"] > 0
+            for k in kernels:
+                res = renderer.render(variant, W, H, SEED_SETS[0], rows=ROWS, kernel=k, sample_block=b, sample_blocks=R, want_accum=True, want_rng=True)
+                what = (variant, nlights, k, b)
+                assert np.array_equal(res.accum[r0:r1].view(np.uint32), ref["accum"][r0:r1].view(np.uint32)), what
+                assert np.array_equal(res.rng_state.reshape(H, W, 4)[r0:r1], ref["rng_state"].reshape(H, W, 4)[r0:r1]), what
+                assert np.array_equal(res.image[r0:r1], ref["image"][r0:r1]), what
+                for c in ("samples", "rays", "shadow_rays"):
+                    assert res.counters[c] == ref["counters"][c], what + (c,)
 
 
 def test_sample_sharding_errors(renderer, scene_dirs):

@@ -12,6 +12,7 @@ from conftest import SEED_SETS
 
 pytestmark = pytest.mark.gpu
 COUNTERS = ("samples", "rays", "shadow_rays", "tri_tests", "prim_tests")
+FIVE_LIGHTS = np.array([[10, 4, 10, 200], [15, 2, 7, 0], [3, -2, 14, 90], [8, 5, 3, 60], [14, 0, 13.5, 300]], np.float32)
 
 
 def _same(res, ref, H, W, rows, what):
@@ -40,22 +41,27 @@ def test_spec_full_frame_bit_exact(renderer, scene_dirs, oracle_fma, oracle_sep,
 
 @pytest.mark.parametrize("spp", [1, 7, 32, 33, 100])
 def test_spec_sample_counts_and_scene_memories(renderer, scene_dirs, oracle_fma, spp):
+    """Sample counts that cut the last batch or window short, with the scene's two lights and with 1 and 5 (odd counts
+    place the window-mode candidates one RNG pair apart instead of two)"""
     d = scene_dirs["torus"]
-    renderer.set_scene(pt.load_scene_dir(d, "base"))
+    scene = pt.load_scene_dir(d, "base")
     osc = oracle_fma.load_scene_dir(d, "base")
     W, H, rows = 512, 512, (140, 172)
-    ref = oracle_fma.render("base", W, H, SEED_SETS[0], osc, spp=spp, rows=rows)
-    for mem in ("smem", "const"):
-        res = renderer.render("base", W, H, SEED_SETS[0], rows=rows, spp=spp, kernel="spec", scene_mem=mem, want_accum=True, want_rng=True)
-        _same(res, ref, H, W, rows, "torus spp %d %s" % (spp, mem))
+    for lights in (scene.lights, FIVE_LIGHTS[:1], FIVE_LIGHTS):
+        scene.lights = osc["lights"] = lights
+        renderer.set_scene(scene)
+        ref = oracle_fma.render("base", W, H, SEED_SETS[0], osc, spp=spp, rows=rows)
+        for mem in ("smem", "const"):
+            res = renderer.render("base", W, H, SEED_SETS[0], rows=rows, spp=spp, kernel="spec", scene_mem=mem, want_accum=True, want_rng=True)
+            _same(res, ref, H, W, rows, "torus spp %d %s %d lights" % (spp, mem, len(lights)))
 
 
 def test_spec_mispredicting_pixels(renderer, oracle_fma):
-    """A mesh far above the floor against the sky: along its silhouette hit and sky samples alternate inside one pixel, so
-    batches are cut at the first surprise and redone; rows through the silhouette must still be bit-exact."""
-    import gen_mesh
-    tris = gen_mesh.soup(400, seed=3, box_lo=8.0, box_size=6.0, edge=(0.5, 0.9))           # sparse cloud of big triangles
-    tris[:, [2, 6, 10]] += 12.0                                                              # lift it above the horizon line
+    """A sparse cloud of big triangles in view and above the horizon, against the sky: along its silhouette hit and sky
+    samples alternate inside one pixel, so batches are cut at the first surprise and redone; rows through the silhouette
+    must still be bit-exact."""
+    from test_light_counts_gpu import silhouette_triangles
+    tris = silhouette_triangles()
     sph, sq = np.zeros(9, np.int32), np.zeros(9, np.int32)
     lights = np.array([[10, 4, 10, 400], [15, 2, 7, 300]], np.float32)
     scene = pt.Scene(sph, sq, tris, lights)
@@ -68,7 +74,10 @@ def test_spec_mispredicting_pixels(renderer, oracle_fma):
     # rows where the mesh is visible against the sky (alpha-independent: colour differs from pure sky rows)
     ref = oracle_fma.render("base", W, H, SEED_SETS[0], osc)
     _same(spec, ref, H, W, (0, H), "silhouette scene")
-    assert spec.counters["tri_tests_executed"] > 0
+    sky = oracle_fma.render("base", W, H, SEED_SETS[0], dict(osc, triangles=tris[:0]), want_accum=False, want_rng=False)
+    assert (ref["image"] != sky["image"]).any()                             # the triangles are in view
+    # SPEC threw speculation away: triangle tests the megakernel never ran
+    assert spec.counters["tri_tests_executed"] > full.counters["tri_tests_executed"] > 0
 
 
 def test_spec_tiles_stripes_and_culls(renderer, scene_dirs):

@@ -183,3 +183,40 @@ def test_cuda_vlpgrid_needs_its_inputs_and_a_fresh_grid(scene_dirs):
         r.set_vpls(vpl)                                                   # a new buffer invalidates the grid
         with pytest.raises(pt.PtError):
             r.render("vlpgrid", 64, 64, (1, 2, 3, 4))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("nlights", [1, 5])
+def test_cuda_vlpgrid_other_light_counts(renderer, scene_dirs, oracle_fma, nlights):
+    """lightTracer -> VLP bounds -> VLP grid -> pathTracer, all on the device, with 1 and 5 lights (n_vlp VPLs per light)"""
+    from test_bidir_gpu import same_floats
+    from test_spec_kernel_gpu import FIVE_LIGHTS
+    scene = pt.load_scene_dir(scene_dirs["bidir"], "bidir")
+    scene.lights = FIVE_LIGHTS[:nlights]
+    renderer.set_scene(scene)
+    osc = oracle_fma.load_scene_dir(scene_dirs["bidir"], "bidir")
+    osc["lights"] = scene.lights
+    seeds, n = FRAME_SEEDS[1], 300
+    renderer.light_tracer(seeds, n)
+    vpl = renderer.read_vpls()
+    ovpl = oracle_fma.light_tracer(seeds, osc, n)
+    assert vpl.shape == (n * nlights, 4) and same_floats(vpl, ovpl)
+    lo, hi = renderer.vlp_bounds()
+    olo, ohi = oracle_fma.vlp_bounds(ovpl)
+    assert np.array_equal(lo.view(np.uint32), olo.view(np.uint32)) and np.array_equal(hi.view(np.uint32), ohi.view(np.uint32))
+    g = pt.vlp_grid_dims(lo, hi, vpl.shape[0], 3.0)
+    renderer.build_vlp_grid(g)
+    start, refs = renderer.read_vlp_grid_csr()
+    ostart, orefs = oracle_fma.build_vlp_grid(ovpl, olo, np.array(g.res[:]), np.array(g.cell_size[:], np.float32))
+    assert np.array_equal(start, ostart) and np.array_equal(refs, orefs)
+    W = H = 512
+    for rows in ((112, 144), (340, 372)):
+        ref = oracle_fma.render("vlpgrid", W, H, seeds, osc, vpls=ovpl, rows=rows)        # grid=None: the reference host's grid
+        res = renderer.render("vlpgrid", W, H, seeds, rows=rows, want_accum=True, want_rng=True)
+        r0, r1 = rows
+        assert np.array_equal(res.image[r0:r1], ref["image"][r0:r1]), (nlights, rows)
+        assert same_floats(res.accum[r0:r1], ref["accum"][r0:r1]), (nlights, rows)
+        assert np.array_equal(res.rng_state.reshape(H, W, 4)[r0:r1], ref["rng_state"].reshape(H, W, 4)[r0:r1]), (nlights, rows)
+        for k in ("samples", "rays", "shadow_rays", "tri_tests", "prim_tests"):
+            assert res.counters[k] == ref["counters"][k], (nlights, rows, k)
+        assert ref["counters"]["shadow_rays"] > 0
