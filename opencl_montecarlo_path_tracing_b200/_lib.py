@@ -140,6 +140,8 @@ PTCUDA_SYMBOLS = {
     "pt_multi_launch_pathtracer": (_VP, [_VP, C.POINTER(pt_camera), C.POINTER(pt_render_params)]),
     "pt_multi_map_render": (_VP, [_VP, C.POINTER(_VP)]),
     "pt_multi_get_counters": (_I, [_VP, C.POINTER(pt_counters)]),
+    "pt_multi_set_bounces": (_I, [_VP, _I]),
+    "pt_set_bounces": (_I, [_VP, _I]),
     "pt_wait": (_I, [_VP]),
     "pt_runtime_ms": (_D, [_VP]),
     "pt_release_event": (None, [_VP]),

@@ -344,10 +344,15 @@ class Renderer:
         _check(self._l.pt_read_vlp_grid_cells(self.ctx, raw.ctypes.data_as(C.c_void_p), ncells), "pt_read_vlp_grid_cells")
         return raw.reshape(ncells, 128)
 
-    def render(self, variant, width, height, seeds, read_image=True, samples=None, **kw):
+    def set_bounces(self, bounces):
+        """Diffuse bounces per path (0..15) for the following renders of this context (pt_set_bounces; DESIGN.md 5b)."""
+        _check(self._l.pt_set_bounces(self.ctx, int(bounces)), "pt_set_bounces")
+
+    def render(self, variant, width, height, seeds, read_image=True, samples=None, bounces=0, **kw):
         """Renders the frame in one launch, or with samples=(b, e) samples [b, e) of it as one range of a progression
         (include/ptcuda.h, "progressive rendering"): the last range gives the one-launch frame bit for bit, earlier ones a
         preview image.  accum / rng_state are read back when want_accum / want_rng are set.
+        bounces: diffuse bounces per path with Russian roulette (include/ptcuda.h, DESIGN.md 5b); 0 is the reference.
 
             kw = dict(spp=256)
             for b, e in ((0, 16), (16, 64), (64, 256)):
@@ -358,6 +363,7 @@ class Renderer:
             out = r2.render("base", 1920, 1080, seeds, samples=(16, 256), **kw)
         """
         p = make_params(variant, width, height, seeds, **kw)
+        self.set_bounces(bounces)
         if samples is None:
             evt = self._l.pt_launch_pathtracer(self.ctx, C.byref(self.cam), C.byref(p))
         else:
@@ -387,7 +393,7 @@ class Renderer:
             res.rng_state = st
         return res
 
-    def set_render_state(self, variant, width, height, seeds, samples_done, accum, rng_state, **kw):
+    def set_render_state(self, variant, width, height, seeds, samples_done, accum, rng_state, bounces=0, **kw):
         """Restores a progression saved after samples_done samples (accum (H, W, 4) float32 and rng_state (H*W, 4) uint32, as
         render(..., samples=(b, samples_done), want_accum=True, want_rng=True) returned them); keywords as for render().  The
         next render(..., samples=(samples_done, e)) with the same params continues it."""
@@ -396,13 +402,15 @@ class Renderer:
         st = np.ascontiguousarray(rng_state, np.uint32)
         if acc.size != width * height * 4 or st.size != width * height * 4:
             raise ValueError("set_render_state: accum and rng_state must hold width * height * 4 values each")
+        self.set_bounces(bounces)
         _check(self._l.pt_set_render_state(self.ctx, C.byref(self.cam), C.byref(p), int(samples_done),
                                            acc.ctypes.data_as(C.POINTER(C.c_float)), st.ctypes.data_as(C.POINTER(C.c_uint32))),
                "pt_set_render_state")
 
-    def render_device(self, variant, width, height, seeds, d_rgba8, d_accum=None, **kw):
+    def render_device(self, variant, width, height, seeds, d_rgba8, d_accum=None, bounces=0, **kw):
         """Render into caller-owned device memory (raw pointers, e.g. torch tensors' data_ptr())."""
         p = make_params(variant, width, height, seeds, **kw)
+        self.set_bounces(bounces)
         _check(self._l.pt_render_device(self.ctx, C.byref(self.cam), C.byref(p), C.c_void_p(d_rgba8),
                                         C.c_void_p(d_accum) if d_accum else None), "pt_render_device")
 

@@ -22,6 +22,8 @@
  *   PT_GPUS=n          render on GPUs 0..n-1 of this box (row stripes + one NCCL reduce of the accumulation buffer)
  *   PT_SHARD=samples   with PT_GPUS=n: shard the SAMPLES of every pixel over the GPUs instead of row stripes (throughput
  *                      mode: other RNG streams per block, statistically equivalent image, not bit-identical)
+ *   PT_BOUNCES=n       base, lmem and trianglegrid: n (0..15) diffuse bounces per path with Russian roulette (include/ptcuda.h
+ *                      pt_set_bounces, DESIGN.md 5b; also with PT_GPUS=n).  Default 0: the reference's image
  *   PT_NO_WARMUP=1     skip the untimed one-row warm-up launch
  *   PT_EXTRA_OUTPUT=png,ppm   additionally write result.png (RGBA PNG) and/or result_p6.ppm (binary P6) next to result.ppm
  *   PT_STATS=1         append Mrays/s, samples/s and work counters after the reference's own lines
@@ -269,6 +271,10 @@ int pth_cli_main(int variant, int argc, char **argv) {
     rp.scene_mem = env_choice("PT_SCENE_MEM", mems, 3, PT_SCENE_AUTO);
     rp.arith = env_choice("PT_ARITH", ariths, 2, PT_ARITH_FMA);
     rp.no_cull = getenv("PT_NO_CULL") ? atoi(getenv("PT_NO_CULL")) : 0;
+    if (!nodof && !bidir && getenv("PT_BOUNCES")) {       /* diffuse bounces per path (0..15, DESIGN.md 5b) */
+        const int nb = atoi(getenv("PT_BOUNCES"));
+        pt_check(multi ? pt_multi_set_bounces(multi, nb) : pt_set_bounces(ctx, nb), "PT_BOUNCES=%s", getenv("PT_BOUNCES"));
+    }
     if (multi && getenv("PT_SHARD") && !strcmp(getenv("PT_SHARD"), "samples")) rp.sample_blocks = ngpus;
 
     pt_event light_evt = NULL;

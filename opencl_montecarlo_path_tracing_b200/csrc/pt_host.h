@@ -65,6 +65,7 @@ struct pt_progression_key {
     uint32_t seeds[4];
     pt_camera cam;
     uint64_t scene_version, grid_version, vpl_version, vlp_grid_version;   // the inputs the variant reads (0: not read)
+    int max_bounces;                                                        // pt_set_bounces
 };
 
 struct pt_ctx_s {
@@ -121,6 +122,9 @@ struct pt_ctx_s {
     int last_kernel;              // PT_KERNEL_* the most recent render resolved to (after PT_KERNEL_AUTO)
     int accum_valid_w, accum_valid_h;   // extent of d_accum the most recent launch wrote (0: it did not request it)
     size_t rng_valid_items;             // work-items of d_rng the most recent launch wrote
+
+    // diffuse bounces per path (pt_set_bounces, DESIGN.md 5b); 0 = the reference's single-vertex sample
+    int max_bounces;
 
     // progressive rendering: d_accum / d_rng hold the state of this progression after its first `prog_next` samples
     bool prog_active;
@@ -189,5 +193,6 @@ int pt_launch_stream_grid(pt_ctx ctx, const pt_render_params *p, const pt::Launc
 int pt_launch_spec(pt_ctx ctx, const pt_render_params *p, const pt::LaunchArgs &args);
 int pt_launch_grid_pool(pt_ctx ctx, const pt_render_params *p, const pt::LaunchArgs &args);
 int pt_launch_bidir(pt_ctx ctx, const pt_render_params *p, const pt::LaunchArgs &args);
+int pt_launch_bounce(pt_ctx ctx, const pt_render_params *p, const pt::LaunchArgs &args, int max_bounces);
 int pt_launch_light_tracer_kernels(pt_ctx ctx, int arith, const pt::LaunchArgs &args, int n, float4 *vpl, uint4 *rng_out,
                                    float4 *active, int *count);

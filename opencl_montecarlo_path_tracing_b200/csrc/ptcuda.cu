@@ -30,6 +30,7 @@
 #include "pt_gridqueue.cuh"
 #include "pt_gridasync.cuh"
 #include "pt_metropolis.cuh"
+#include "pt_bounce.cuh"
 
 // ------------------------------------------------------------------------------------ errors
 static std::atomic<int> g_error_mode{PT_ERRORS_EXIT};
@@ -568,6 +569,13 @@ static int validate_params(pt_ctx c, const pt_render_params *p) {
     }
     if ((long long)p->width * p->height * (p->variant == PT_VARIANT_NODOF ? 64 : 1) > 0x7fffffffLL)
         return pt_fail(1, "render: work-item ids exceed 31 bits (the reference computes them in int)");
+    if (c->max_bounces > 0) {
+        if (p->variant != PT_VARIANT_BASE && p->variant != PT_VARIANT_LMEM && p->variant != PT_VARIANT_GRID)
+            return pt_fail(1, "render: diffuse bounces (pt_set_bounces %d) are defined for the base, lmem and trianglegrid variants only", c->max_bounces);
+        if (p->kernel != PT_KERNEL_MEGA && p->kernel != PT_KERNEL_AUTO)
+            return pt_fail(1, "render: diffuse bounces (pt_set_bounces %d) run in the per-pixel kernel only (PT_KERNEL_MEGA / AUTO), not flavour %d",
+                           c->max_bounces, p->kernel);
+    }
     return 0;
 }
 
@@ -733,7 +741,8 @@ static pt_render_params resolve_auto(pt_ctx c, const pt_render_params *in, const
     const int nrows = A.nrows;
     pt_render_params p = *in;
     if (p.kernel == PT_KERNEL_AUTO) {
-        if (p.variant == PT_VARIANT_BIDIR || p.variant == PT_VARIANT_VLPGRID) p.kernel = PT_KERNEL_MEGA;
+        if (c->max_bounces > 0) p.kernel = PT_KERNEL_MEGA;             // k_bounce_pixel: the one flavour that traces paths
+        else if (p.variant == PT_VARIANT_BIDIR || p.variant == PT_VARIANT_VLPGRID) p.kernel = PT_KERNEL_MEGA;
         else if (p.variant == PT_VARIANT_NODOF) p.kernel = PT_KERNEL_MEGA;   // single-copy Sample(): 0.433 ms vs 0.479 ms persistent (512x512)
         else if (p.variant == PT_VARIANT_GRID) p.kernel = PT_KERNEL_MEGA;
         else {
@@ -764,6 +773,7 @@ static int dispatch(pt_ctx c, const pt_render_params *p, const pt::LaunchArgs &A
         if (p->kernel != PT_KERNEL_MEGA) return pt_fail(1, "render: the bidirectional variants have the megakernel flavour only (PT_KERNEL_MEGA / AUTO)");
         return pt_launch_bidir(c, p, A);
     }
+    if (c->max_bounces > 0) return pt_launch_bounce(c, p, A, c->max_bounces);     // validate_params: MEGA, base / lmem / grid
     switch (p->kernel) {
         case PT_KERNEL_MEGA: return pt_launch_mega(c, p, A);
         case PT_KERNEL_PERSISTENT: return pt_launch_persistent(c, p, A);
@@ -802,6 +812,7 @@ static int progression_params(pt_ctx c, const pt_camera *cam, const pt_render_pa
     if (p->variant == PT_VARIANT_GRID) key->grid_version = c->grid_version;
     if (p->variant == PT_VARIANT_BIDIR || p->variant == PT_VARIANT_VLPGRID) key->vpl_version = c->vpl_version;
     if (p->variant == PT_VARIANT_VLPGRID) key->vlp_grid_version = c->vlp_grid_version;
+    key->max_bounces = c->max_bounces;
     return 0;
 }
 
@@ -1263,6 +1274,13 @@ __global__ void __launch_bounds__(256) k_peak_issue(unsigned *out, int trips, fl
 // out[2] = warp instructions per second of the mixed FP32 + integer kernel (G), out[3] = its duration in ms
 extern "C" int pt_last_kernel(pt_ctx c) { return c ? c->last_kernel : -1; }
 
+extern "C" int pt_set_bounces(pt_ctx c, int max_bounces) {
+    if (!c) return pt_fail(1, "pt_set_bounces: null context");
+    if (max_bounces < 0 || max_bounces > PT_MAX_BOUNCES) return pt_fail(1, "pt_set_bounces: %d outside [0, %d]", max_bounces, PT_MAX_BOUNCES);
+    c->max_bounces = max_bounces;
+    return 0;
+}
+
 // diagnostics: copy `bytes` of the context's scratch buffer (offset 256: per-CTA timing table of PT_CTA_TIMES=1) to the host
 extern "C" int pt_debug_read_scratch(pt_ctx c, void *dst, size_t offset, size_t bytes) {
     if (!c || !dst || offset + bytes > c->scratch_cap) return pt_fail(1, "pt_debug_read_scratch: out of range");
@@ -1531,6 +1549,16 @@ extern "C" pt_event pt_multi_launch_pathtracer(pt_multi m, const pt_camera *cam,
     c0->accum_valid_w = c0->accum_valid_h = 0; c0->rng_valid_items = 0;
     m->last_w = params->width; m->last_h = params->height;
     return e;
+}
+
+extern "C" int pt_multi_set_bounces(pt_multi m, int max_bounces) {
+    if (!m) return pt_fail(1, "pt_multi_set_bounces: null argument");
+    if (max_bounces < 0 || max_bounces > PT_MAX_BOUNCES) return pt_fail(1, "pt_multi_set_bounces: %d outside [0, %d]", max_bounces, PT_MAX_BOUNCES);
+    for (int i = 0; i < m->n; ++i) {
+        const int rc = pt_set_bounces(m->ctx[i], max_bounces);
+        if (rc) return rc;
+    }
+    return 0;
 }
 
 extern "C" void *pt_multi_map_render(pt_multi m, pt_event *evt) {
